@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the active-perception observation path (see DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one full environment step of the hot path over a batch of synthetic frames that
 is already resident in HBM: ingest (gray/RGB -> resize -> 2-frame max -> ring push) followed by
@@ -167,12 +167,10 @@ _W = {}
 
 
 def reference_root():
-    """Where the UNMODIFIED reference package can be imported from: baseline/_ref (pip-installed copy that travels to
-    the GPU box) or /root/reference (build container).  None = not available: the port is timed instead."""
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isfile(os.path.join(cand, "active_gym", "fov_env.py")):
-            return cand
-    return None
+    """Where the UNMODIFIED reference package can be imported from ($AGYM_REFERENCE_ROOT, else oracle/_ref; see oracle/ref_harness.py).
+    None = not available: the port is timed instead."""
+    from oracle import ref_harness as rh
+    return rh.REFERENCE_ROOT if rh.reference_available() else None
 
 
 class RealReferenceEnv:
@@ -298,7 +296,7 @@ class CpuReference:
 
     def describe(self):
         if self.kind == "reference":
-            return "the unmodified reference (baseline/_ref: fov_env.py + atari_env.py / dmc_env.py) under oracle/ref_harness.py's fake simulators"
+            return "the unmodified reference ($AGYM_REFERENCE_ROOT: fov_env.py + atari_env.py / dmc_env.py) under oracle/ref_harness.py's fake simulators"
         return "oracle/ref_port.py (the reference's per-env cv2 / numpy / torchvision call sequence)"
 
     def close(self):
@@ -452,6 +450,17 @@ class Workload:
         self.ingest()
         self.observe()
         self.t += 1
+
+    def outputs(self, sample=256, seed=0):
+        """What a caller of the step received from the last one, for a fixed seeded sample of envs (the full observation
+        batch is up to 462 MB): observation, fovea location and, for the flexible fovea, its window size; as float arrays."""
+        idx = np.sort(np.random.default_rng(seed).choice(self.n, min(sample, self.n), replace=False))
+        sel = self.torch.from_numpy(idx).to(self.device)
+        d = {"env_index": idx.astype(np.float64), "obs": self.out.index_select(0, sel).float().cpu().numpy(),
+             "fov_loc": self.path.loc.index_select(0, sel).double().cpu().numpy()}
+        if self.w["wrapper"] == "flexible":
+            d["fov_res"] = self.path.res.index_select(0, sel).double().cpu().numpy()
+        return d
 
     def free(self):
         self.frames = self.actions = self.atypes = self.out = self.path = None
@@ -734,8 +743,9 @@ def strong_scaling(torch, dist, device, world, global_envs=16384, instances=8, r
             "l2": f"{ws:.0f} MB of frames / ring / output per GPU over {instances} rotated env batches vs 126 MB L2"}
 
 
-def measure_device(torch, dist, device, world, wname, n, steps, warmup, peak, peak_src, traffic_db, no_graph=False):
-    """Device-timed step (inputs resident in HBM), per-kernel times and the roofline of one workload."""
+def measure_device(torch, dist, device, world, wname, n, steps, warmup, peak, peak_src, traffic_db, no_graph=False, dump=False):
+    """Device-timed step (inputs resident in HBM), per-kernel times and the roofline of one workload.  With `dump`, the
+    result carries `Workload.outputs()` of the last timed step under "outputs"."""
     wl = Workload(wname, device, n=n)
     w = wl.w
     bytes_ = algorithmic_bytes(w)
@@ -751,6 +761,8 @@ def measure_device(torch, dist, device, world, wname, n, steps, warmup, peak, pe
     out = {"config": config_for(wname, wl.n, world), "value": total_envs * steps / dt, "unit": UNIT, "steps": steps,
            "ms_per_step": dt / steps * 1e3, "ms_per_step_eager": dt_eager / steps * 1e3, "launch": launch,
            "gpu_launches": steps * wl.launches_per_step}
+    if dump:   # now: the per-kernel timing below steps the state further
+        out["outputs"] = wl.outputs()
     kern = {}
     reps = max(steps, 10)
     for kname, fn, nb in (("ingest", wl.ingest, bytes_["ingest"]), ("observe", wl.observe, bytes_["observe"])):
@@ -845,7 +857,12 @@ def run_b200_arm(a):
 
     clocks = ClockSampler(local)
     clocks.start()
-    main, wl = measure_device(torch, dist, device, world, a.workload, a.envs, a.steps, a.warmup, peak, peak_src, traffic_db, a.no_graph)
+    main, wl = measure_device(torch, dist, device, world, a.workload, a.envs, a.steps, a.warmup, peak, peak_src, traffic_db, a.no_graph,
+                              dump=a.dump_outputs is not None)
+    if a.dump_outputs is not None and rank == 0:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in main.pop("outputs").items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     # the timed region is only tens of milliseconds: keep the same step loop running (untimed) until the
     # sampler has had about half a second under identical load, so that the clock record means something
     t_load = time.perf_counter()
@@ -910,6 +927,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="time the eager launch loop only (default: the timed steps are captured in a CUDA graph; the eager time is reported next to it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of --workload returned (observation, fov_loc, fov_res for the flexible "
+                         "fovea; 256 sampled envs, indices in env_index) as DIR/<name>.npy in float32 / float64")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
     quiet_stdout()

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE — generates tests/golden/*.npz from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the reference package (see oracle/ref_harness.py):
 
-    python oracle/make_golden.py
+    AGYM_REFERENCE_ROOT=<reference checkout> python oracle/make_golden.py
 
 The reference's fov_env.py / atari_env.py / dmc_env.py are imported as they are, under
 the simulator stubs of oracle/ref_harness.py, and driven through their public

@@ -1,9 +1,10 @@
 """TEST INFRASTRUCTURE — runs the UNMODIFIED reference under simulator stubs.
 
-Only usable in the build container (``/root/reference`` does not exist on the GPU
-box).  It is used by ``oracle/make_golden.py`` to generate the committed fixtures in
-``tests/golden/`` and by ``tests/test_oracle_vs_reference.py`` (skipped when the
-reference is absent) to pin the restated oracle against the reference itself.
+Only usable where a checkout of the reference package (elicassion/active-gym, the
+directory that holds ``active_gym/fov_env.py``) is named by ``AGYM_REFERENCE_ROOT`` or sits
+in the git-ignored ``oracle/_ref/``; the repository does not contain it.  It is used by ``oracle/make_golden.py`` to generate the
+committed fixtures in ``tests/golden/`` and by ``tests/test_oracle_vs_reference.py``
+(skipped when the reference is absent) to pin the restated oracle against the reference itself.
 
 What is stubbed (absent third-party modules, SURVEY.md §8c): ``gymnasium``
 (``Env``/``Wrapper``/``spaces``), ``atari_py`` (``ALEInterface`` replaced by a fake
@@ -20,7 +21,7 @@ import types
 
 import numpy as np
 
-REFERENCE_ROOT = os.environ.get("AGYM_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("AGYM_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def reference_available() -> bool:

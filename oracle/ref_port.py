@@ -1,8 +1,8 @@
 """TEST / BASELINE INFRASTRUCTURE — the reference's per-environment CPU path, restated.
 
 ``bench.py`` times this module as the CPU baseline (``cpu_baseline.kind = "port"`` and the
-``--impl reference`` arm): ``/root/reference`` does not exist on the GPU box, so the
-reference's own files cannot be imported there.  This port performs, per environment and
+``--impl reference`` arm) wherever there is no checkout of the reference (see oracle/ref_harness.py),
+whose own files are then not importable.  This port performs, per environment and
 per step, the same library calls in the same order and dtypes as the reference does —
 ``cv2.resize(INTER_LINEAR)``, ``astype(float32)/255``, a float64 two-frame max, a
 ``deque`` + ``np.stack`` frame stack, ``np.rint(np.clip())`` for the fovea location, NumPy

@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AGYM_LIB") or os.path.join(_HERE, "lib", "libagym_b200.so")  # AGYM_LIB: timing experiments only
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 # status codes / flags (mirrors of the header's macros)
 OK = 0
@@ -39,7 +39,7 @@ class Config(C.Structure):
         ("raw_h", C.c_int32), ("raw_w", C.c_int32), ("raw_c", C.c_int32), ("luma_w", C.c_int32 * 3),
         ("fov_h", C.c_int32), ("fov_w", C.c_int32), ("periph_h", C.c_int32), ("periph_w", C.c_int32),
         ("relative", C.c_int32), ("act_lo", C.c_double), ("act_hi", C.c_double), ("fov_init_loc", C.c_double * 2),
-        ("no_antialias", C.c_int32),
+        ("no_antialias", C.c_int32), ("obs_c", C.c_int32),
     ]
 
 

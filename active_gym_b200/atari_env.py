@@ -39,7 +39,7 @@ class AtariEnvArgs:
             self.__setattr__(k, v)
 
 
-def _path_from_args(args, num_envs, obs_size, raw_shape, luma, device, host_source: bool) -> PipelinedPath:
+def _path_from_args(args, num_envs, obs_size, raw_shape, luma, device, host_source: bool, channels: int = 1) -> PipelinedPath:
     """The per-GPU engine of an env batch.  ``args.shards`` (default: 2 for host frame sources, whose copies should
     overlap the kernels and the copies back; 1 for device-resident sources) cuts the batch into env-index shards with
     their own streams (pipeline.PipelinedPath).  Few, large copies win: a process has 8 hardware work queues by
@@ -58,7 +58,7 @@ def _path_from_args(args, num_envs, obs_size, raw_shape, luma, device, host_sour
         sensory_action_space=getattr(args, "sensory_action_space", (0.0, 0.0)),
         peripheral_res=getattr(args, "peripheral_res", None), device=device,
         cache_peripheral=getattr(args, "cache_peripheral", True), side_streams=host_source,
-        antialias=bool(getattr(args, "antialias", True)))
+        antialias=bool(getattr(args, "antialias", True)), **({"channels": channels} if channels != 1 else {}))
 
 
 class _VecBase(Env):
@@ -67,7 +67,7 @@ class _VecBase(Env):
     alternately — the simulators of one group step on the host while the other group's frames are copied and
     transformed on the GPU (SURVEY.md §8f row 1)."""
 
-    def _init_engine(self, args, num_envs, source, luma, device):
+    def _init_engine(self, args, num_envs, source, luma, device, channels: int = 1):
         self.args = args
         self.num_envs = int(num_envs)
         self.frame_stack = args.frame_stack
@@ -81,12 +81,14 @@ class _VecBase(Env):
         self.source = source
         host_source = not hasattr(source, "device")
         self.path = _path_from_args(args, self.num_envs, self.obs_size, tuple(source.raw_shape), luma,
-                                    device or getattr(args, "device", None), host_source)
+                                    device or getattr(args, "device", None), host_source, channels)
         self.device = self.path.device
         self.host_obs = bool(getattr(args, "host_obs", False))
         if host_source and hasattr(source, "set_used_rows") and self.path.run is not None:
             source.set_used_rows(self.path.used_rows)   # only the sampled raw rows cross PCIe, as one block per shard
-        self.observation_space = Box(low=-1., high=1., shape=(self.frame_stack,) + self.obs_size, dtype=np.float32)
+        # RGB: (K, 3, H, W) as dmc_env.py:122 declares
+        frame_axes = (self.frame_stack,) if channels == 1 else (self.frame_stack, channels)
+        self.observation_space = Box(low=-1., high=1., shape=frame_axes + self.obs_size, dtype=np.float32)
         self._pending = None
         # args.async_sim: step_async hands the simulator stepping (host CPU) + the enqueueing of copies and kernels to a
         # worker thread and returns at once; step_wait joins it.  The caller's thread is free while the simulators run

@@ -87,11 +87,18 @@ int validate(const agym_config &c) {
         if (c.relative && !(c.act_lo <= c.act_hi)) return AGYM_ERR_INVALID_ARG;
     }
     if (c.periph_h > 0 && c.fov_h == 0) return AGYM_ERR_INVALID_ARG;
+    // RGB observations: the render's channels as planes, so only DMC frames rendered at obs_size qualify
+    if (c.obs_c != 0 && c.obs_c != 1 && c.obs_c != 3) return AGYM_ERR_INVALID_ARG;
+    if (c.obs_c == 3 && (c.raw_c != 3 || c.raw_h != c.obs_h || c.raw_w != c.obs_w)) return AGYM_ERR_INVALID_ARG;
     // word/vector granularity the kernels are written for (84x84 obs, 210x160 raw satisfy all)
     if (c.obs_w % 4 != 0 || (c.obs_h * c.obs_w) % 16 != 0) return AGYM_ERR_UNSUPPORTED;
     if (c.obs_h > 255 || c.obs_w > 255 || c.raw_h > 4096 || c.raw_w > 4096) return AGYM_ERR_UNSUPPORTED;
     return AGYM_OK;
 }
+
+inline int planes_per_frame(const agym_config &c) { return c.obs_c == 3 ? 3 : 1; }
+// ring planes per env: frame_stack * C
+inline size_t ring_planes(const agym_config &c) { return static_cast<size_t>(c.frame_stack) * planes_per_frame(c); }
 
 inline cudaStream_t as_stream(void *s) { return reinterpret_cast<cudaStream_t>(s); }
 inline int ret(cudaError_t e) { return e == cudaSuccess ? AGYM_OK : static_cast<int>(e); }
@@ -334,7 +341,7 @@ int agym_plan_create(const agym_config *cfg, agym_plan **out_plan) {
     const uint32_t *base = static_cast<const uint32_t *>(pl->pool);
     DevPlan &d = pl->dev;
     std::memset(&d, 0, sizeof(d));
-    d.N = c.n_envs; d.K = c.frame_stack; d.S_h = c.obs_h; d.S_w = c.obs_w; d.plane = c.obs_h * c.obs_w;
+    d.N = c.n_envs; d.C = planes_per_frame(c); d.K = c.frame_stack * d.C; d.S_h = c.obs_h; d.S_w = c.obs_w; d.plane = c.obs_h * c.obs_w;
     d.raw_h = c.raw_h; d.raw_w = c.raw_w; d.raw_c = c.raw_c;
     d.lw0 = c.luma_w[0]; d.lw1 = c.luma_w[1]; d.lw2 = c.luma_w[2];
     d.f_h = c.fov_h; d.f_w = c.fov_w; d.p_h = c.periph_h; d.p_w = c.periph_w;
@@ -429,11 +436,11 @@ int agym_plan_destroy(agym_plan *plan) {
 }
 
 size_t agym_plan_ring_bytes(const agym_plan *plan) {
-    return plan ? static_cast<size_t>(plan->cfg.n_envs) * plan->cfg.frame_stack * plan->cfg.obs_h * plan->cfg.obs_w : 0;
+    return plan ? static_cast<size_t>(plan->cfg.n_envs) * ring_planes(plan->cfg) * plan->cfg.obs_h * plan->cfg.obs_w : 0;
 }
 
 size_t agym_plan_pcache_bytes(const agym_plan *plan) {
-    return plan ? sizeof(float) * static_cast<size_t>(plan->cfg.n_envs) * plan->cfg.frame_stack * plan->cfg.periph_h *
+    return plan ? sizeof(float) * static_cast<size_t>(plan->cfg.n_envs) * ring_planes(plan->cfg) * plan->cfg.periph_h *
                       plan->cfg.periph_w
                 : 0;
 }
@@ -442,6 +449,7 @@ int agym_ingest_atari(const agym_plan *plan, const uint8_t *d_frames_a, const ui
                       const uint8_t *d_flags, uint8_t *d_ring, int32_t *d_head, float *d_pcache, void *stream) {
     if (!plan || !d_frames_a || !d_frames_b || !d_flags || !d_ring || !d_head) return AGYM_ERR_INVALID_ARG;
     if (d_pcache && plan->cfg.periph_h == 0) return AGYM_ERR_INVALID_ARG;
+    if (plan->dev.C != 1) return AGYM_ERR_UNSUPPORTED;            // ALE's grey screen is the only Atari observation
     if (plan->cfg.raw_w % 16 != 0) return AGYM_ERR_UNSUPPORTED;  // rows are staged as 16-byte vectors
     return ret(launch_ingest_atari(plan->dev, d_frames_a, d_frames_b, d_flags, d_ring, d_head, d_pcache, as_stream(stream)));
 }
@@ -460,6 +468,7 @@ int agym_ingest_atari_packed(const agym_plan *plan, const uint8_t *d_rows_a, con
                              const uint8_t *d_flags, uint8_t *d_ring, int32_t *d_head, float *d_pcache, void *stream) {
     if (!plan || !d_rows_a || !d_rows_b || !d_flags || !d_ring || !d_head) return AGYM_ERR_INVALID_ARG;
     if (d_pcache && plan->cfg.periph_h == 0) return AGYM_ERR_INVALID_ARG;
+    if (plan->dev.C != 1) return AGYM_ERR_UNSUPPORTED;
     if (plan->cfg.raw_w % 16 != 0) return AGYM_ERR_UNSUPPORTED;
     return ret(launch_ingest_atari(plan->dev_packed, d_rows_a, d_rows_b, d_flags, d_ring, d_head, d_pcache, as_stream(stream)));
 }
@@ -501,7 +510,7 @@ int agym_observe_fixed(const agym_plan *plan, const uint8_t *d_ring, const int32
     if (v != AGYM_OK) return v;
     if (variant < AGYM_OUT_CROP || variant > AGYM_OUT_RESIZE_FULL) return AGYM_ERR_INVALID_ARG;
     const agym_config &c = plan->cfg;
-    const size_t bytes = static_cast<size_t>(c.n_envs) * c.frame_stack * (variant == AGYM_OUT_CROP ? c.fov_h * c.fov_w : c.obs_h * c.obs_w);
+    const size_t bytes = static_cast<size_t>(c.n_envs) * ring_planes(c) * (variant == AGYM_OUT_CROP ? c.fov_h * c.fov_w : c.obs_h * c.obs_w);
     if ((v = check_norm_args(d_out, bytes, d_out_norm, norm_dtype)) != AGYM_OK) return v;
     return ret(launch_observe_fixed(plan->dev, d_ring, d_head, d_action, d_fov_ctrl, d_loc, variant, d_out, d_out_norm, norm_dtype,
                                     as_stream(stream)));
@@ -514,7 +523,7 @@ int agym_observe_peripheral(const agym_plan *plan, const uint8_t *d_ring, const 
     if (v != AGYM_OK) return v;
     if (plan->cfg.periph_h == 0) return AGYM_ERR_INVALID_ARG;
     const agym_config &c = plan->cfg;
-    if ((v = check_norm_args(d_out, static_cast<size_t>(c.n_envs) * c.frame_stack * c.obs_h * c.obs_w, d_out_norm, norm_dtype)) != AGYM_OK) return v;
+    if ((v = check_norm_args(d_out, static_cast<size_t>(c.n_envs) * ring_planes(c) * c.obs_h * c.obs_w, d_out_norm, norm_dtype)) != AGYM_OK) return v;
     return ret(launch_observe_peripheral(plan->dev, &plan->expand_std, d_ring, d_head, d_pcache, d_action, d_fov_ctrl, d_loc, d_out,
                                          d_out_norm, norm_dtype, as_stream(stream)));
 }
@@ -527,7 +536,7 @@ int agym_observe_flexible(const agym_plan *plan, const uint8_t *d_ring, const in
     if (!d_res || variant < AGYM_OUT_CROP || variant > AGYM_OUT_RESIZE_FULL) return AGYM_ERR_INVALID_ARG;
     if (variant == AGYM_OUT_CROP && (pad_h <= 0 || pad_w <= 0 || pad_w % 4 != 0)) return AGYM_ERR_INVALID_ARG;
     const agym_config &c = plan->cfg;
-    const size_t bytes = static_cast<size_t>(c.n_envs) * c.frame_stack *
+    const size_t bytes = static_cast<size_t>(c.n_envs) * ring_planes(c) *
                          (variant == AGYM_OUT_CROP ? static_cast<size_t>(pad_h) * pad_w : static_cast<size_t>(c.obs_h) * c.obs_w);
     if ((v = check_norm_args(d_out, bytes, d_out_norm, norm_dtype)) != AGYM_OK) return v;
     return ret(launch_observe_flexible(plan->dev, d_ring, d_head, d_action, d_atype, d_fov_ctrl, d_loc, d_res, variant,

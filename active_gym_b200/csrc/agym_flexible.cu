@@ -639,8 +639,12 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
         const size_t tile = (size_t)p.K * oh * ow;
         const size_t fixed = a16(tile + 4 * (size_t)p.K * p.S_h * (p.S_w / 4 + 2)) +
                              4 * ((size_t)p.S_w * 8 + 2 * (size_t)p.S_h * p.blur_tmax + p.S_w + p.S_h) + 16;
-        const size_t budget = 114000;  // + static shared memory + 1 KB reserved per CTA: two CTAs per SM (233,472 B)
         const size_t one = (size_t)p.S_h * (p.S_w + 4), all = (size_t)p.K * one;   // floats: one / all K frames of the largest window
+        // + static shared memory + 1 KB reserved per CTA: two CTAs per SM (233,472 B).  RGB plans whose fixed buffers do
+        // not leave one window's t1 in that budget (mask_out at 3 frames x 3 planes: 133 KB of tile and strips) run
+        // one CTA per SM with the whole SM's shared memory instead
+        const int ctas_per_sm = (p.C == 3 && fixed + 4 * one > 114000) ? 1 : 2;
+        const size_t budget = ctas_per_sm == 2 ? 114000 : 225000;
         const size_t room = budget > fixed ? ((budget - fixed) / 4) & ~size_t(3) : 0;
         const size_t t1_cap = std::min(all, room);
         if (tile % 16 == 0 && ow % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && t1_cap >= one &&
@@ -650,7 +654,7 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
             int dev = 0, sms = 148;
             cudaGetDevice(&dev);
             cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            const int grid = std::min(p.N, 2 * sms);
+            const int grid = std::min(p.N, ctas_per_sm * sms);
             // the env-claim counter starts every launch at zero (stream-ordered; a launch that faulted cannot leave it armed)
             if ((e = cudaMemsetAsync(p.flex_counters, 0, 16, st)) != cudaSuccess) return e;
             if (variant == AGYM_OUT_CROP) {

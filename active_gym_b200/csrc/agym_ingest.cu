@@ -673,6 +673,102 @@ __global__ void __launch_bounds__(kThreads) k_ingest_dmc(const __grid_constant__
     }
 }
 
+// ---------------------------------------------------------------------- ingest: DMC, RGB
+// 16 interleaved 3-channel pixels (48 bytes, 12 words) -> the 16 bytes of each channel plane.  Output word m of
+// channel c holds bytes c, 3+c, 6+c, 9+c of the 12-byte run w[3m .. 3m+2]: two PRMTs per word, no arithmetic.
+__device__ __forceinline__ void split_rgb16(const uint32_t (&w)[12], uint4 &r, uint4 &g, uint4 &b) {
+    uint32_t o[3][4];
+#pragma unroll
+    for (int m = 0; m < 4; ++m) {
+        const uint32_t w0 = w[3 * m], w1 = w[3 * m + 1], w2 = w[3 * m + 2];
+        o[0][m] = __byte_perm(__byte_perm(w0, w1, 0x0630), w2, 0x5210);   // bytes 0, 3, 6 | 9
+        o[1][m] = __byte_perm(__byte_perm(w0, w1, 0x0741), w2, 0x6210);   // bytes 1, 4, 7 | 10
+        o[2][m] = __byte_perm(__byte_perm(w0, w1, 0x0052), w2, 0x7410);   // bytes 2, 5 | 8, 11
+    }
+    r = make_uint4(o[0][0], o[0][1], o[0][2], o[0][3]);
+    g = make_uint4(o[1][0], o[1][1], o[1][2], o[1][3]);
+    b = make_uint4(o[2][0], o[2][1], o[2][2], o[2][3]);
+}
+
+// DMCEnv._get_obs pixel branch with grey=False + stack logic (dmc_env.py:122, 175-183, 228-230): the render's three
+// channels, unconverted, pushed as the three planes of the next frame slot (head indexes planes, see the header).
+// Same structure and flag semantics as k_ingest_dmc; the luma is replaced by a byte split.
+__global__ void __launch_bounds__(kThreads) k_ingest_dmc_rgb(const __grid_constant__ DevPlan p,
+                                                             const uint8_t *__restrict__ f, const uint8_t *__restrict__ flags,
+                                                             uint8_t *__restrict__ ring, int32_t *__restrict__ head,
+                                                             float *__restrict__ pcache) {
+    constexpr int C = 3;
+    extern __shared__ __align__(16) uint8_t smem[];
+    const int n = blockIdx.x, tid = threadIdx.x;
+    const uint8_t *src = f + (size_t)n * p.plane * 3;
+    const int nvec = p.plane / 16;
+    // as in k_ingest_dmc: the first two groups are requested before flags / head are known
+    uint32_t w0[12], w1[12];
+    const int t0 = tid, t1 = tid + kThreads;
+    if (t0 < nvec) {
+        const uint8_t *q = src + (size_t)t0 * 48;
+        *reinterpret_cast<uint4 *>(w0) = ld_stream128(q);
+        *reinterpret_cast<uint4 *>(w0 + 4) = ld_stream128(q + 16);
+        *reinterpret_cast<uint4 *>(w0 + 8) = ld_stream128(q + 32);
+    }
+    if (t1 < nvec) {
+        const uint8_t *q = src + (size_t)t1 * 48;
+        *reinterpret_cast<uint4 *>(w1) = ld_stream128(q);
+        *reinterpret_cast<uint4 *>(w1 + 4) = ld_stream128(q + 16);
+        *reinterpret_cast<uint4 *>(w1 + 8) = ld_stream128(q + 32);
+    }
+    const int fl = flags[n];
+    const int hd = head[n];
+    if (fl & AGYM_FLAG_IDLE) return;
+    const int frames = p.K / C;
+    const int slot = hd / C + 1 == frames ? 0 : hd / C + 1;
+    const int plane0 = C * slot;   // planes plane0 .. plane0 + 2 receive R, G, B
+    const size_t vpp = (size_t)p.plane / 16;
+    uint8_t *s_frame = smem;       // [C][plane] when the cache is refreshed
+    float *s_t1 = reinterpret_cast<float *>(smem + C * align16(p.plane));
+    __syncthreads();
+    if (tid == 0) head[n] = plane0 + C - 1;
+
+    uint4 *dst = reinterpret_cast<uint4 *>(ring + ((size_t)n * p.K + plane0) * p.plane);
+    uint4 *s4 = reinterpret_cast<uint4 *>(s_frame);
+    const size_t svp = align16(p.plane) / 16;
+    auto put = [&](int t, const uint32_t (&w)[12]) {
+        uint4 r, g, b;
+        split_rgb16(w, r, g, b);
+        dst[t] = r; dst[vpp + t] = g; dst[2 * vpp + t] = b;
+        if (pcache) { s4[t] = r; s4[svp + t] = g; s4[2 * svp + t] = b; }
+    };
+    if (t0 < nvec) put(t0, w0);
+    if (t1 < nvec) put(t1, w1);
+    for (int t = tid + 2 * kThreads; t < nvec; t += kThreads) {  // larger observations
+        uint32_t w[12];
+        const uint8_t *q = src + (size_t)t * 48;
+        *reinterpret_cast<uint4 *>(w) = ld_stream128(q);
+        *reinterpret_cast<uint4 *>(w + 4) = ld_stream128(q + 16);
+        *reinterpret_cast<uint4 *>(w + 8) = ld_stream128(q + 32);
+        put(t, w);
+    }
+    if (fl & AGYM_FLAG_HARD_RESET) {
+        for (int k = 0; k < p.K; ++k) {
+            if (k >= plane0 && k < plane0 + C) continue;
+            uint4 *z = reinterpret_cast<uint4 *>(ring + ((size_t)n * p.K + k) * p.plane);
+            for (int i = tid; i < p.plane / 16; i += kThreads) z[i] = make_uint4(0u, 0u, 0u, 0u);
+            if (pcache) {
+                float *zc = pcache + ((size_t)n * p.K + k) * p.p_h * p.p_w;
+                for (int i = tid; i < p.p_h * p.p_w; i += kThreads) zc[i] = 0.f;
+            }
+        }
+    }
+    if (pcache) {
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+            __syncthreads();   // c = 0: the staged planes are complete; c > 0: the previous H pass has read s_t1
+            squeeze_to_cache(p, s_frame + c * align16(p.plane), s_t1,
+                             pcache + ((size_t)n * p.K + plane0 + c) * p.p_h * p.p_w, tid, kThreads);
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------- stack
 // np.stack(state_buffer) (atari_env.py:143, dmc_env.py:230): oldest -> newest.
 __global__ void __launch_bounds__(kThreads) k_stack(const __grid_constant__ DevPlan p, const uint8_t *__restrict__ ring,
@@ -822,8 +918,14 @@ cudaError_t launch_ingest_atari(const DevPlan &p, const uint8_t *fa, const uint8
 
 cudaError_t launch_ingest_dmc(const DevPlan &p, const uint8_t *f, const uint8_t *flags, uint8_t *ring, int32_t *head,
                               float *pcache, cudaStream_t st) {
-    size_t smem = pcache ? a16(p.plane) + sizeof(float) * p.S_h * p.p_w : 0;
     cudaError_t e;
+    if (p.C == 3) {   // RGB plan: three planes per push, one CTA per env as below
+        const size_t smem = pcache ? 3 * a16(p.plane) + sizeof(float) * p.S_h * p.p_w : 0;
+        if ((e = set_smem(k_ingest_dmc_rgb, smem)) != cudaSuccess) return e;
+        k_ingest_dmc_rgb<<<p.N, kThreads, smem, st>>>(p, f, flags, ring, head, pcache);
+        return cudaGetLastError();
+    }
+    size_t smem = pcache ? a16(p.plane) + sizeof(float) * p.S_h * p.p_w : 0;
     if ((e = set_smem(k_ingest_dmc, smem)) != cudaSuccess) return e;
     // plain launch: programmatic dependent launch (launch_pdl) was measured slower for this grid of 8,192 short CTAs —
     // the next kernel's CTAs, let in early, sit blocked on the SM slots the later waves need (DMC step 0.071 - 0.099 ms

@@ -20,7 +20,8 @@ struct FlexEntry {
 };
 
 struct DevPlan {
-    int32_t N, K, S_h, S_w, plane;      // plane = S_h * S_w
+    int32_t N, K, S_h, S_w, plane;      // plane = S_h * S_w; K = ring planes per env = frame_stack * C
+    int32_t C;                          // planes per frame: 1 grey, 3 RGB (ring layout: include/agym_b200.h)
     int32_t raw_h, raw_w, raw_c;
     int32_t lw0, lw1, lw2;              // luma weights per channel position
     int32_t f_h, f_w, p_h, p_w;

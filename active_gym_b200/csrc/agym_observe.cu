@@ -222,7 +222,7 @@ __global__ void __launch_bounds__(kCropWarps * 32) k_observe_fixed_crop_v2(const
 // its own index arithmetic), (ii) a lane assembles the output words of a GROUP of g rows (g * f_w bytes = whole words:
 // g = 1, 2 or 4) by funnel-shifting the aligned words of each row — one LDS + one SHF per output word instead of a table
 // load, four byte loads and three PRMTs — and parks them in a shared-memory tile that holds the CTA's envs back to back,
-// (iii) the tile leaves as ONE TMA bulk store per CTA (8 envs are a multiple of 16 bytes whatever the window), or as
+// (iii) the tile leaves as ONE TMA bulk store per CTA (4 or 8 envs are a multiple of 16 bytes whatever the window), or as
 // coalesced words from the last, partial CTA.  F_W != 0 fixes the window width at compile time (every loop unrolls, no
 // per-word bookkeeping); F_W == 0 is the same code for any width.  Measured (DESIGN.md 3.5): the crop is bound by its
 // scattered 64-byte DRAM granules, not by instructions — v3 is 4-9 % faster than v2 away from 8,192 envs, equal there.
@@ -233,8 +233,8 @@ struct CropV3Args {
     int slice;              // staged bytes per warp (incl. 16 spare bytes in front)
 };
 constexpr int kCrop3Warps = 8;
-template <int F_W>
-__global__ void __launch_bounds__(kCrop3Warps * 32) k_observe_fixed_crop_v3(const __grid_constant__ DevPlan p,
+template <int F_W, int WARPS = kCrop3Warps>   // WARPS: envs per CTA
+__global__ void __launch_bounds__(WARPS * 32) k_observe_fixed_crop_v3(const __grid_constant__ DevPlan p,
                                                                             const uint8_t *__restrict__ ring,
                                                                             const int32_t *__restrict__ head,
                                                                             const double *__restrict__ action,
@@ -243,7 +243,7 @@ __global__ void __launch_bounds__(kCrop3Warps * 32) k_observe_fixed_crop_v3(cons
                                                                             const CropV3Args a) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int n = blockIdx.x * kCrop3Warps + warp;
+    const int n = blockIdx.x * WARPS + warp;
     const bool valid = n < p.N;
     const int fw = F_W ? F_W : p.f_w;
     const int nch = F_W ? (F_W + 30) / 16 : a.nch;
@@ -251,7 +251,7 @@ __global__ void __launch_bounds__(kCrop3Warps * 32) k_observe_fixed_crop_v3(cons
     const int gw = g * fw / 4;
     const int K = p.K, rows = K * p.f_h, stride = nch * 16, out_env = rows * fw, words = out_env >> 2;
     uint8_t *s_in = smem + (size_t)warp * a.slice + 16;   // [rows][stride]; 16 spare bytes in front (a row's first word may start 3 bytes early)
-    uint32_t *s_tile = reinterpret_cast<uint32_t *>(smem + (size_t)kCrop3Warps * a.slice);   // [envs of the CTA][words]
+    uint32_t *s_tile = reinterpret_cast<uint32_t *>(smem + (size_t)WARPS * a.slice);   // [envs of the CTA][words]
     uint32_t *s_out = s_tile + warp * words;
     if (valid) {
         LocIn li;
@@ -343,13 +343,13 @@ __global__ void __launch_bounds__(kCrop3Warps * 32) k_observe_fixed_crop_v3(cons
             }
         }
     }
-    const int n0 = blockIdx.x * kCrop3Warps;
-    const bool bulk = n0 + kCrop3Warps <= p.N && (reinterpret_cast<uintptr_t>(out) & 15) == 0;   // uniform over the CTA
+    const int n0 = blockIdx.x * WARPS;
+    const bool bulk = n0 + WARPS <= p.N && (reinterpret_cast<uintptr_t>(out) & 15) == 0;   // uniform over the CTA
     if (bulk) {
         fence_async_smem();
         __syncthreads();
         if (threadIdx.x == 0) {
-            bulk_s2g(out + (size_t)n0 * out_env, s_tile, (uint32_t)(kCrop3Warps * out_env));
+            bulk_s2g(out + (size_t)n0 * out_env, s_tile, (uint32_t)(WARPS * out_env));
             bulk_commit();
         }
     } else if (valid) {
@@ -927,19 +927,26 @@ cudaError_t launch_observe_fixed(const DevPlan &p0, const uint8_t *ring, const i
     c3.ngroups = p.K * p.f_h / c3.g;
     c3.m_fh = 0xFFFFFFFFu / (uint32_t)p.f_h + 1u;
     c3.slice = (int)(16 + (size_t)p.K * p.f_h * c3.nch * 16);
-    const size_t crop3_smem = (size_t)kCrop3Warps * (c3.slice + (size_t)p.K * p.f_h * p.f_w);
+    // RGB plans stage three times the planes per env (K = 9 at frame_stack 3: 8 envs x 21,076 B for f = 30 is past the
+    // cap), so they run the same kernel with four envs per CTA (84,304 B); grey plans keep eight
+    const int c3_warps = (p.C == 3 && (size_t)kCrop3Warps * (c3.slice + (size_t)p.K * p.f_h * p.f_w) > 100 * 1024) ? 4 : kCrop3Warps;
+    const size_t crop3_smem = (size_t)c3_warps * (c3.slice + (size_t)p.K * p.f_h * p.f_w);
     if (variant == AGYM_OUT_CROP && (p.K * p.f_h * p.f_w) % 4 == 0 && (p.K * p.f_h) % c3.g == 0 && p.plane % 16 == 0 &&
         (reinterpret_cast<uintptr_t>(ring) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 3) == 0 &&
         !g_disable_std && !g_crop_old && !g_crop_v2 && crop3_smem <= 100 * 1024) {
-        const int grid = (p.N + kCrop3Warps - 1) / kCrop3Warps;
+        const int grid = (p.N + c3_warps - 1) / c3_warps;
         // (plain launch: see launch_ingest_dmc about programmatic dependent launch and multi-wave grids)
-        if (p.f_w == 30) {
-            if ((e = set_smem(k_observe_fixed_crop_v3<30>, crop3_smem)) != cudaSuccess) return e;
-            k_observe_fixed_crop_v3<30><<<grid, kCrop3Warps * 32, crop3_smem, st>>>(p, ring, head, action, ctrl, loc, out, c3);
-        } else {
-            if ((e = set_smem(k_observe_fixed_crop_v3<0>, crop3_smem)) != cudaSuccess) return e;
-            k_observe_fixed_crop_v3<0><<<grid, kCrop3Warps * 32, crop3_smem, st>>>(p, ring, head, action, ctrl, loc, out, c3);
-        }
+#define AGYM_LAUNCH_CROP3(FW, W)                                                                                  \
+    {                                                                                                             \
+        if ((e = set_smem(k_observe_fixed_crop_v3<FW, W>, crop3_smem)) != cudaSuccess) return e;                   \
+        k_observe_fixed_crop_v3<FW, W><<<grid, W * 32, crop3_smem, st>>>(p, ring, head, action, ctrl, loc, out, c3); \
+    }
+        if (c3_warps == 4) {
+            if (p.f_w == 30) AGYM_LAUNCH_CROP3(30, 4)
+            else AGYM_LAUNCH_CROP3(0, 4)
+        } else if (p.f_w == 30) AGYM_LAUNCH_CROP3(30, kCrop3Warps)
+        else AGYM_LAUNCH_CROP3(0, kCrop3Warps)
+#undef AGYM_LAUNCH_CROP3
         return cudaGetLastError();   // the normalised output, if any, was written by the kernel
     }
     if (variant == AGYM_OUT_CROP && (p.K * p.f_h * p.f_w) % 4 == 0 && !g_disable_std && !g_crop_old &&
@@ -1034,6 +1041,7 @@ cudaError_t launch_observe_peripheral(const DevPlan &p0, const ExpandStd *ew, co
     }
         if (p.K == 4 && p.plane == 7056) AGYM_LAUNCH_PF(4, 1764)
         else if (p.K == 3 && p.plane == 7056) AGYM_LAUNCH_PF(3, 1764)
+        else if (p.C == 3 && p.K % 3 == 0 && p.plane == 7056) AGYM_LAUNCH_PF(3, 1764)   // RGB: 3 frames x 3 planes
         else if (p.K % 4 == 0) AGYM_LAUNCH_PF(4, 0)
         else if (p.K % 3 == 0) AGYM_LAUNCH_PF(3, 0)
         else if (p.K % 2 == 0) AGYM_LAUNCH_PF(2, 0)

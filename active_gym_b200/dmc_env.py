@@ -1,9 +1,15 @@
 """DeepMind-Control base env: ``DMCEnvArgs``, the batched ``DMCVecEnv`` and the factories.
 
-Mirrors the pixel / grey branch of ``active_gym/dmc_env.py`` (citations refer to it).  MuJoCo
-physics and rendering stay on the host (``sources.DMCPool``); luma + frame stack + the foveal
-wrappers run on the GPU.  ``from_pixels=False`` and ``grey=False`` are outside the hot path
-(the latter is shape-inconsistent in the reference, dmc_env.py:122 vs :230) and raise.
+Mirrors the pixel branch of ``active_gym/dmc_env.py`` (citations refer to it).  MuJoCo
+physics and rendering stay on the host (``sources.DMCPool``); luma (``grey=True``) or the
+channel split (``grey=False``) + frame stack + the foveal wrappers run on the GPU.
+``from_pixels=False`` is outside the hot path and raises.
+
+``grey=False`` observations have the layout the reference declares, ``(K, 3, H, W)`` (dmc_env.py:122;
+its stacking at :230 is of HWC frames, inconsistent with that declaration): oldest frame first, each frame
+the render's channels in render order (RGB), unconverted.  The foveal wrappers act on the last two axes of
+every one of the 3K planes with one fov_loc / fov_res per env, as fov_env.py's slicing and Resize do on any
+array with leading axes.
 """
 from __future__ import annotations
 
@@ -42,16 +48,17 @@ class DMCEnvArgs:
 
 
 class DMCVecEnv(_VecBase):
-    """N DMC environments; observation = (N, K, S_h, S_w) uint8 CUDA tensor (dmc_env.py:78-253)."""
+    """N DMC environments; observation = (N, K, S_h, S_w) uint8 CUDA tensor, or (N, K, 3, S_h, S_w) with
+    ``grey=False`` (dmc_env.py:78-253)."""
 
     def __init__(self, args, num_envs: int = 1, source=None, device=None):
-        if not args.from_pixels or not args.grey:
-            raise NotImplementedError("only the from_pixels=True, grey=True branch is on the observation hot path")
+        if not args.from_pixels:
+            raise NotImplementedError("only the from_pixels=True branch is on the observation hot path")
         if source is None:
             from .sources import DMCPool
             source = DMCPool(args, int(num_envs), workers=getattr(args, "sim_workers", 1))
         # dmc_env.py:182 applies COLOR_BGR2GRAY to an RGB render: channel 0 gets the blue weight
-        self._init_engine(args, num_envs, source, LUMA_DMC, device)
+        self._init_engine(args, num_envs, source, LUMA_DMC, device, channels=1 if args.grey else 3)
         self._true_low, self._true_high = source.true_low, source.true_high
         self.action_space = Box(low=-1.0, high=1.0, shape=self._true_low.shape, dtype=np.float32)  # dmc_env.py:110-115
 

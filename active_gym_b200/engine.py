@@ -40,8 +40,12 @@ class ObservationPath:
                  fov_init_loc: Sequence[float] = (0, 0), sensory_action_mode: str = "absolute",
                  sensory_action_space: Sequence[float] = (0.0, 0.0), peripheral_res: Optional[Tuple[int, int]] = None,
                  device: Optional[torch.device] = None, cache_peripheral: bool = True, buffers: Optional[dict] = None,
-                 antialias: bool = True):
-        """``antialias``: how the wrappers' ``torchvision.transforms.Resize`` calls (fov_env.py:120, 248, 366-368) are
+                 antialias: bool = True, channels: int = 1):
+        """``channels``: planes per frame — 1 (grey, the luma of the frames) or 3 (RGB: the channels of DMC renders,
+        which must have ``raw_shape == obs_size + (3,)``).  The ring then holds ``frame_stack * channels`` planes
+        (``include/agym_b200.h``) and every observation gains a channel axis, ``(N, K, C, h, w)``.
+
+        ``antialias``: how the wrappers' ``torchvision.transforms.Resize`` calls (fov_env.py:120, 248, 366-368) are
         restated — antialiased bilinear (the installed torchvision's default, what the fixtures were recorded with) or
         plain bilinear (the default of older torchvision releases on tensors; SURVEY.md section 8c)."""
         if not torch.cuda.is_available():
@@ -55,6 +59,9 @@ class ObservationPath:
         if sensory_action_mode not in ("absolute", "relative"):
             raise ValueError(f"sensory_action_mode must be 'absolute' or 'relative', got {sensory_action_mode!r}")
         self.relative = sensory_action_mode == "relative"
+        if channels not in (1, 3):
+            raise ValueError(f"channels must be 1 (grey) or 3 (RGB), got {channels!r}")
+        self.channels = int(channels)
         cfg = _lib.Config()
         cfg.n_envs, cfg.frame_stack = self.n_envs, self.frame_stack
         cfg.obs_h, cfg.obs_w = self.obs_size
@@ -69,13 +76,14 @@ class ObservationPath:
         cfg.act_lo, cfg.act_hi = lo, hi
         cfg.fov_init_loc[:] = [float(fov_init_loc[0]), float(fov_init_loc[1])]
         cfg.no_antialias = 0 if antialias else 1
+        cfg.obs_c = self.channels
         self.antialias = bool(antialias)
         self._cfg = cfg
         self._L = _lib.lib()
         self._plan = C.c_void_p()
         with torch.cuda.device(self.device):
             _lib.check(self._L.agym_plan_create(C.byref(cfg), C.byref(self._plan)), "agym_plan_create")
-        N, K, (S_h, S_w) = self.n_envs, self.frame_stack, self.obs_size
+        N, K, (S_h, S_w) = self.n_envs, self.frame_stack * self.channels, self.obs_size   # K: ring planes
         dev = self.device
         if buffers is not None:
             # slices of a larger batch owned by the caller (PipelinedPath): contiguous, already initialised
@@ -187,20 +195,29 @@ class ObservationPath:
 
     # ------------------------------------------------------------------ outputs
     def stack(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """np.stack(state_buffer), oldest -> newest (atari_env.py:143, dmc_env.py:230)."""
+        """np.stack(state_buffer), oldest -> newest (atari_env.py:143, dmc_env.py:230): (N, K, S_h, S_w), or
+        (N, K, C, S_h, S_w) for RGB (a view of the plane stack the kernel writes)."""
         if out is None:
             out = torch.empty_like(self.ring)
         with torch.cuda.device(self.device):
             _lib.check(self._L.agym_stack(self._plan, _ptr(self.ring), _ptr(self.head), _ptr(out), self._stream()), "agym_stack")
-        return out
+        return out.view(self.stack_shape)
+
+    @property
+    def stack_shape(self) -> Tuple[int, ...]:
+        return (self.n_envs,) + self._frame_axes() + self.obs_size
+
+    def _frame_axes(self) -> Tuple[int, ...]:
+        """(K,) for grey, (K, C) for RGB: the planes of the ring in observation order."""
+        return (self.frame_stack,) if self.channels == 1 else (self.frame_stack, self.channels)
 
     def out_shape(self, kind: str, variant: str, pad: Optional[Tuple[int, int]] = None) -> Tuple[int, ...]:
-        N, K, S = self.n_envs, self.frame_stack, self.obs_size
+        NK, S = (self.n_envs,) + self._frame_axes(), self.obs_size
         if kind == "peripheral" or variant in ("mask", "resize_full"):
-            return (N, K) + S
+            return NK + S
         if kind == "flexible":
-            return (N, K) + tuple(pad if pad is not None else S)
-        return (N, K) + self.fov_size
+            return NK + tuple(pad if pad is not None else S)
+        return NK + self.fov_size
 
     def _ctrl(self, ctrl) -> Optional[torch.Tensor]:
         if ctrl is None:

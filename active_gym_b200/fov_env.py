@@ -170,7 +170,8 @@ class RecordWrapper(Wrapper):
 
 class FixedFovealEnv(Wrapper):
     """fov_env.py:107-234 for N envs.  Observation: uint8 CUDA tensor (N, K, f_h, f_w), or
-    (N, K, S_h, S_w) with ``mask_out`` / ``resize_to_full``."""
+    (N, K, S_h, S_w) with ``mask_out`` / ``resize_to_full``; RGB base envs (DMC ``grey=False``) add a channel axis
+    after K, (N, K, 3, h, w)."""
 
     _kind = "fixed"
 
@@ -201,7 +202,7 @@ class FixedFovealEnv(Wrapper):
             "sensory_action": Box(low=self.sensory_action_space[0], high=self.sensory_action_space[1], dtype=int),
         })
         shape = self.obs_size if (self.mask_out or self.resize) else self.fov_size
-        self.observation_space = Box(low=-1., high=1., shape=(self.env.frame_stack,) + tuple(shape), dtype=np.float32)
+        self.observation_space = Box(low=-1., high=1., shape=self._frame_axes() + tuple(shape), dtype=np.float32)
         self._rec = self.env if isinstance(self.env, RecordWrapper) else None
         self._obs = None
         self._host = None
@@ -214,9 +215,14 @@ class FixedFovealEnv(Wrapper):
         self.last_obs_u8 = None
         self._out = None          # set_output(): where the observe kernels store the u8 observations
 
+    def _frame_axes(self):
+        """(K,) or, for RGB, (K, 3): the axes in front of the two pixel axes."""
+        c = getattr(self.path, "channels", 1)
+        return (self.env.frame_stack,) if c == 1 else (self.env.frame_stack, c)
+
     @property
     def obs_shape(self):
-        """Shape of the batched u8 observation tensor, (N, K, h, w)."""
+        """Shape of the batched u8 observation tensor, (N, K, h, w) or (N, K, 3, h, w)."""
         return tuple(self.path.out_shape(self._kind, self.variant))
 
     def set_output(self, out: Optional[torch.Tensor]) -> None:
@@ -396,7 +402,7 @@ class FixedFovealPeripheralEnv(FixedFovealEnv):
         self.mask_out = False
         self.resize_to_full = True
         self.peripheral_res = tuple(args.peripheral_res)
-        self.observation_space = Box(low=-1., high=1., shape=(self.env.frame_stack,) + tuple(self.obs_size), dtype=np.float32)
+        self.observation_space = Box(low=-1., high=1., shape=self._frame_axes() + tuple(self.obs_size), dtype=np.float32)
         if self.path.peripheral_res != self.peripheral_res:
             raise ValueError("the base env was built from different args (peripheral_res mismatch)")
 
@@ -436,7 +442,7 @@ class SingleEnvAdapter:
         o = obs[0].cpu().numpy()
         if getattr(self.env, "_kind", "") == "flexible" and self.env.variant == "crop":
             rh, rw = self.fov_res
-            o = o[:, :rh, :rw]
+            o = o[..., :rh, :rw]
         return (o.astype(np.float32) / np.float32(255.0)).astype(np.float64)
 
     @staticmethod

@@ -84,7 +84,7 @@ class PipelinedPath:
     def __init__(self, n_envs: int, frame_stack: int, obs_size, raw_shape, shards: int = 1, device=None,
                  luma: Sequence[int] = LUMA_RGB, fov_size=None, fov_init_loc=(0, 0), sensory_action_mode: str = "absolute",
                  sensory_action_space=(0.0, 0.0), peripheral_res=None, cache_peripheral: bool = True,
-                 packed_h2d: bool = True, side_streams: bool = False, antialias: bool = True):
+                 packed_h2d: bool = True, side_streams: bool = False, antialias: bool = True, channels: int = 1):
         if not torch.cuda.is_available():
             raise RuntimeError("active_gym_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
@@ -94,7 +94,9 @@ class PipelinedPath:
         self.fov_size = None if fov_size is None else (int(fov_size[0]), int(fov_size[1]))
         self.peripheral_res = None if peripheral_res is None else (int(peripheral_res[0]), int(peripheral_res[1]))
         self.relative = sensory_action_mode == "relative"
-        N, K, (S_h, S_w), dev = self.n_envs, self.frame_stack, self.obs_size, self.device
+        self.channels = int(channels)
+        # K: ring planes per env (frame_stack * channels, see ObservationPath)
+        N, K, (S_h, S_w), dev = self.n_envs, self.frame_stack * self.channels, self.obs_size, self.device
         shards = max(1, min(int(shards), N))
         self.ranges: List[Tuple[int, int]] = [r for r in all_shards(N, shards) if r[1] > r[0]]
         with torch.cuda.device(dev):
@@ -112,10 +114,10 @@ class PipelinedPath:
             self.ep_len = torch.zeros((N,), dtype=torch.int64, device=dev)
             self.cum_reward = torch.zeros((N,), dtype=torch.float64, device=dev)
             self.paths = [
-                ObservationPath(hi - lo, K, self.obs_size, self.raw_shape, luma=luma, fov_size=fov_size,
+                ObservationPath(hi - lo, self.frame_stack, self.obs_size, self.raw_shape, luma=luma, fov_size=fov_size,
                                 fov_init_loc=fov_init_loc, sensory_action_mode=sensory_action_mode,
                                 sensory_action_space=sensory_action_space, peripheral_res=peripheral_res, device=dev,
-                                cache_peripheral=cache_peripheral, antialias=antialias,
+                                cache_peripheral=cache_peripheral, antialias=antialias, channels=self.channels,
                                 buffers=dict(ring=self.ring[lo:hi], head=self.head[lo:hi], loc=self.loc[lo:hi],
                                              res=self.res[lo:hi], pcache=None if self.pcache is None else self.pcache[lo:hi],
                                              err=self.err))
@@ -152,6 +154,10 @@ class PipelinedPath:
 
     def out_shape(self, kind: str, variant: str, pad=None) -> Tuple[int, ...]:
         return (self.n_envs,) + tuple(self.paths[0].out_shape(kind, variant, pad)[1:])
+
+    @property
+    def stack_shape(self) -> Tuple[int, ...]:
+        return (self.n_envs,) + tuple(self.paths[0].stack_shape[1:])
 
     def reset_counters(self) -> None:
         self.h2d_bytes = self.d2h_bytes = 0
@@ -357,7 +363,7 @@ class PipelinedPath:
         for i, lo, hi in self._shards():
             self.paths[i].stack(out=out[lo:hi])
         self.join()
-        return out
+        return out.view(self.stack_shape)
 
     def _observe(self, kind: str, action, action_type, variant: str, ctrl, pad, out, host_out: bool, norm_out=None):
         shape = self.out_shape(kind, variant, pad)

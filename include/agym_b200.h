@@ -22,13 +22,21 @@
  *   - u8 pixels everywhere: the reference's normalised float value is
  *     float64(float32(u)/255) for the u8 value u (SURVEY.md §8).
  *
- * Data layout in HBM (N = envs, K = frame_stack, S = obs_size, f = fov_size)
- *   ring  u8  [N][K][S_h][S_w]  frame stack; slot head[n] holds the NEWEST frame, logical
- *                               order oldest->newest is (head+1)%K ... head
+ * Data layout in HBM (N = envs, K = frame_stack, C = obs_c planes per frame, P = K * C planes,
+ * S = obs_size, f = fov_size)
+ *   ring  u8  [N][P][S_h][S_w]  frame stack as a stack of P planes; head[n] is the plane index of the
+ *                               NEWEST plane, logical order oldest->newest is (head+1)%P ... head.
+ *                               Grey (C = 1): one plane per frame, head = slot of the newest frame.
+ *                               RGB (C = 3): a frame occupies the C planes C*s .. C*s+C-1 of slot s (R, G, B),
+ *                               and head = C*s + C-1 for the newest slot s; a push writes slot
+ *                               s' = (head/C + 1) % K and sets head = (head + C) % P.  Read oldest->newest,
+ *                               the planes are frame-major and channel-minor: the layout (K, C, S_h, S_w).
  *   head  i32 [N]
  *   loc   i32 [N][2]            (row, col) of the fovea's upper-left corner
  *   res   i32 [N][2]            (rows, cols) of the flexible fovea
- *   pcache f32 [N][K][p_h][p_w] optional cache of each ring slot's peripheral squeeze
+ *   pcache f32 [N][P][p_h][p_w] optional cache of each ring plane's peripheral squeeze
+ * Every observe call works plane by plane with one fov_loc / fov_res per env, so its outputs below are
+ * written with P planes in place of K: (N, K, C, h, w) in memory.
  */
 #ifndef AGYM_B200_H
 #define AGYM_B200_H
@@ -40,7 +48,7 @@
 extern "C" {
 #endif
 
-#define AGYM_ABI_VERSION 3
+#define AGYM_ABI_VERSION 4
 
 #if defined(__GNUC__)
 #define AGYM_API __attribute__((visibility("default")))
@@ -102,6 +110,8 @@ typedef struct agym_config {
     double fov_init_loc[2];      /* fov_init_loc (fov_env.py:111,149-150)                      */
     int32_t no_antialias;        /* 0: torchvision Resize as installed today (antialias=True, fov_env.py:120,248,366-368);
                                     1: plain bilinear, the default of older torchvision releases on tensors     */
+    int32_t obs_c;               /* planes per observed frame: 0 or 1 = grey (luma, dmc_env.py:182); 3 = RGB, the render's
+                                    channels unconverted (DMC only: raw_c == 3 and raw == obs; dmc_env.py:122)         */
 } agym_config;
 
 typedef struct agym_plan agym_plan;   /* opaque: validated config + device coefficient tables */
@@ -121,7 +131,8 @@ AGYM_API size_t agym_plan_pcache_bytes(const agym_plan *plan);
 /* Replaces AtariEnv._get_state + the frame logic of _step/_reset (atari_env.py:73-75,
  * 80-82, 91, 111-114, 121-133): per env gray(A),gray(B) -> cv2 INTER_LINEAR resize to
  * obs_size -> max -> push into the ring.  d_frames_a / d_frames_b: u8 [N][raw_h][raw_w][raw_c].
- * d_pcache (may be NULL): also refresh the pushed slot's peripheral squeeze cache. */
+ * d_pcache (may be NULL): also refresh the pushed slot's peripheral squeeze cache.
+ * Grey plans only (obs_c 0 / 1): AGYM_ERR_UNSUPPORTED on an RGB plan, as for the _packed variant. */
 AGYM_API int agym_ingest_atari(const agym_plan *plan, const uint8_t *d_frames_a, const uint8_t *d_frames_b,
                       const uint8_t *d_flags, uint8_t *d_ring, int32_t *d_head, float *d_pcache,
                       void *stream);
@@ -136,13 +147,15 @@ AGYM_API int agym_ingest_atari_packed(const agym_plan *plan, const uint8_t *d_ro
                              const uint8_t *d_flags, uint8_t *d_ring, int32_t *d_head, float *d_pcache,
                              void *stream);
 
-/* Replaces DMCEnv._get_obs (pixel, grey branch) + stack logic (dmc_env.py:175-183, 193-195,
- * 206-207, 228-230): luma of the rendered frame -> push.  d_frames: u8 [N][S_h][S_w][3]. */
+/* Replaces DMCEnv._get_obs (pixel branch) + stack logic (dmc_env.py:175-183, 193-195,
+ * 206-207, 228-230): luma of the rendered frame (grey plan) or its three channels as three planes
+ * (RGB plan, see the ring layout) -> push.  d_frames: u8 [N][S_h][S_w][3].  A hard reset zeroes every
+ * plane except the ones just pushed, and their cache entries. */
 AGYM_API int agym_ingest_dmc(const agym_plan *plan, const uint8_t *d_frames, const uint8_t *d_flags,
                     uint8_t *d_ring, int32_t *d_head, float *d_pcache, void *stream);
 
 /* Replaces np.stack(state_buffer) (atari_env.py:143, dmc_env.py:230): the base env's
- * observation, oldest -> newest.  d_out: u8 [N][K][S_h][S_w]. */
+ * observation, oldest -> newest.  d_out: u8 [N][K * C][S_h][S_w]. */
 AGYM_API int agym_stack(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head, uint8_t *d_out,
                void *stream);
 

@@ -18,7 +18,7 @@ ABI_VERSION = 4
 OK = 0
 FLAG_FRAME_A, FLAG_FRAME_B, FLAG_HARD_RESET, FLAG_IDLE = 1, 2, 4, 8
 FOV_APPLY, FOV_RESET, FOV_KEEP = 0, 1, 2
-OUT_CROP, OUT_MASK, OUT_RESIZE_FULL = 0, 1, 2
+OUT_CROP, OUT_MASK, OUT_RESIZE_FULL, OUT_RESIZE_FOV = 0, 1, 2, 3
 ATYPE_FOV_LOC, ATYPE_FOV_RES = 0, 1
 ERR_RES_RANGE, ERR_RES_FRACTION = 1, 2
 DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2

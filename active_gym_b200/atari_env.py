@@ -35,6 +35,8 @@ class AtariEnvArgs:
         self.record = False
         self.clip_reward = False
         self.resize_to_full = False  # superset: no default in the reference (fov_env.py:120)
+        # superset: FlexibleFovealEnv returns the glimpse, the window resampled to fov_size (N, K, f_h, f_w)
+        self.resize_to_fov = False
         for k, v in kwargs.items():
             self.__setattr__(k, v)
 

@@ -161,7 +161,7 @@ int agym_plan_create(const agym_config *cfg, agym_plan **out_plan) {
     const int s_max = c.obs_h > c.obs_w ? c.obs_h : c.obs_w;
     size_t o_flex = 0, o_flexb = 0, o_flexq = 0, o_flexh2 = 0, o_counters = 0;
     bool have_flexq = false;
-    int blur_tmax = 0;
+    int blur_tmax = 0, fov_tmax = 0;
     if (c.fov_h > 0) {
         full_w = add_axis(pool, c.fov_w, c.obs_w, aa); full_h = add_axis(pool, c.fov_h, c.obs_h, aa);
         // flexible fovea: for every window size r, r->f, f->r and r->S on both axes
@@ -174,6 +174,7 @@ int agym_plan_create(const agym_config *cfg, agym_plan **out_plan) {
                     const AxisOff a = add_axis(pool, n_in, n_out, aa);
                     int32_t *e = index.data() + (static_cast<size_t>(axis * 3 + fam) * (s_max + 1) + r) * 4;
                     e[0] = static_cast<int32_t>(a.xmin); e[1] = static_cast<int32_t>(a.w); e[2] = a.taps; e[3] = a.n_out;
+                    if (fam == 0) fov_tmax = std::max(fov_tmax, a.taps);
                 }
         }
         o_flex = pool.add_i(index);
@@ -361,6 +362,7 @@ int agym_plan_create(const agym_config *cfg, agym_plan **out_plan) {
         d.flex = reinterpret_cast<const FlexEntry *>(base + o_flex);
         d.flexb = reinterpret_cast<const FlexEntry *>(base + o_flexb);
         d.blur_tmax = blur_tmax;
+        d.fov_tmax = fov_tmax;
         d.flexq = have_flexq ? reinterpret_cast<const FlexEntry *>(base + o_flexq) : nullptr;
         d.flexh2 = have_flexq ? reinterpret_cast<const FlexEntry *>(base + o_flexh2) : nullptr;
         d.flex_counters = have_flexq ? reinterpret_cast<int32_t *>(static_cast<uint32_t *>(pl->pool) + o_counters) : nullptr;
@@ -533,11 +535,13 @@ int agym_observe_flexible(const agym_plan *plan, const uint8_t *d_ring, const in
                           int pad_h, int pad_w, uint8_t *d_out, int32_t *d_err, void *d_out_norm, int norm_dtype, void *stream) {
     int v = check_fov_args(plan, d_ring, d_head, d_action, d_fov_ctrl, d_loc, d_out);
     if (v != AGYM_OK) return v;
-    if (!d_res || variant < AGYM_OUT_CROP || variant > AGYM_OUT_RESIZE_FULL) return AGYM_ERR_INVALID_ARG;
+    if (!d_res || variant < AGYM_OUT_CROP || variant > AGYM_OUT_RESIZE_FOV) return AGYM_ERR_INVALID_ARG;
     if (variant == AGYM_OUT_CROP && (pad_h <= 0 || pad_w <= 0 || pad_w % 4 != 0)) return AGYM_ERR_INVALID_ARG;
     const agym_config &c = plan->cfg;
     const size_t bytes = static_cast<size_t>(c.n_envs) * ring_planes(c) *
-                         (variant == AGYM_OUT_CROP ? static_cast<size_t>(pad_h) * pad_w : static_cast<size_t>(c.obs_h) * c.obs_w);
+                         (variant == AGYM_OUT_CROP         ? static_cast<size_t>(pad_h) * pad_w
+                          : variant == AGYM_OUT_RESIZE_FOV ? static_cast<size_t>(c.fov_h) * c.fov_w
+                                                           : static_cast<size_t>(c.obs_h) * c.obs_w);
     if ((v = check_norm_args(d_out, bytes, d_out_norm, norm_dtype)) != AGYM_OK) return v;
     return ret(launch_observe_flexible(plan->dev, d_ring, d_head, d_action, d_atype, d_fov_ctrl, d_loc, d_res, variant,
                                        pad_h, pad_w, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));

@@ -73,7 +73,7 @@ __global__ void __launch_bounds__(kThreads) k_observe_flexible(const __grid_cons
             bufA[i] = (float)__ldg(src + (r0 + y) * p.S_w + c0 + x);
         }
         __syncthreads();
-        if (blur) {  // Resize(fov_size) then Resize(fov_res) (fov_env.py:276-280)
+        if (blur && VARIANT != AGYM_OUT_RESIZE_FOV) {  // Resize(fov_size) then Resize(fov_res) (fov_env.py:276-280)
             resample_w<float>(bufA, rw, bufB, p.f_w, rh, flex_axis(p, 1, 0, rw, rw), tid, kThreads);
             __syncthreads();
             resample_h<float>(bufB, p.f_w, bufA, p.f_w, p.f_w, flex_axis(p, 0, 0, rh, rh), tid, kThreads);
@@ -84,7 +84,16 @@ __global__ void __launch_bounds__(kThreads) k_observe_flexible(const __grid_cons
             __syncthreads();
         }
         uint32_t *dst = reinterpret_cast<uint32_t *>(out + ((size_t)n * p.K + k) * oh * ow);
-        if (VARIANT == AGYM_OUT_RESIZE_FULL) {
+        if (VARIANT == AGYM_OUT_RESIZE_FOV) {
+            // Resize(fov_size) of the unblurred window (fov_env.py:248,284-285), written byte by byte: a plane of
+            // f_h * f_w bytes need not start on a word (the (21, 33) fovea, an output view at an odd address)
+            resample_w<float>(bufA, rw, bufB, p.f_w, rh, flex_axis(p, 1, 0, rw, rw), tid, kThreads);
+            __syncthreads();
+            resample_h<float>(bufB, p.f_w, bufA, p.f_w, p.f_w, flex_axis(p, 0, 0, rh, rh), tid, kThreads);
+            __syncthreads();
+            uint8_t *d8 = out + ((size_t)n * p.K + k) * p.f_h * p.f_w;
+            for (int i = tid; i < p.f_h * p.f_w; i += kThreads) d8[i] = (uint8_t)quant_u8(bufA[i]);
+        } else if (VARIANT == AGYM_OUT_RESIZE_FULL) {
             resample_w<float>(bufA, rw, bufB, p.S_w, rh, flex_axis(p, 1, 2, rw, rw), tid, kThreads);
             __syncthreads();
             const AxisRef ah = flex_axis(p, 0, 2, rh, rh);
@@ -274,6 +283,11 @@ __global__ void __launch_bounds__(kThreads) k_observe_flexible_fast(const __grid
 // from the fp64 weights: 0.01 LSB for the 5-tap operators of windows up to 50).  Along H it is packed
 // fp32 (FFMA2) on four columns per thread; results are rounded to nearest-even with the 1.5 * 2^23 bias
 // and leave as whole words.
+// VARIANT AGYM_OUT_RESIZE_FOV (the glimpse, Resize(fov_size) of the unblurred window, fov_env.py:248,284-285) reuses
+// the claims, the fov update, the strip copies and the operator prefetch; its two passes (rw -> f_w, then rh -> f_h)
+// are fp32 with the r -> f tables of family 0, evaluated in the order of the table-driven kernel (bit-identical to it).
+// The tile is K * f_h * f_w bytes with no zero fill; a tile that is not a multiple of 16 bytes (f_w = 30 at K = 3 or
+// K * C = 9) or a 16-byte-misaligned output leaves as 4-byte words from the worker threads instead of the bulk store.
 #ifndef AGYM_FLEX_THREADS
 #define AGYM_FLEX_THREADS 256
 #endif
@@ -377,6 +391,39 @@ __device__ __forceinline__ void flex_wpass(const uint32_t *xrow0, int rh, int ro
     }
 }
 
+// Glimpse W pass over nrows staged rows (row r = row r % rh of frame r / rh): t1[r][x] = sum_t w[x][t] * X[r][c0 + xw[x] + t]
+// for the f_w output columns, fp32 in the tap order of resample_w.
+__device__ __forceinline__ void glimpse_wpass(const uint32_t *xrow0, int rh, int S_w, int strip_w, const int32_t *s_xw,
+                                              const float *s_ww, int tw, float *s_t1, int f_w, int c0, int nrows, int tid,
+                                              const uint32_t *s_magic) {
+    const FastDiv fd_fw(f_w, s_magic), fd_rh(rh, s_magic);
+    for (int i = tid; i < nrows * f_w; i += kFlexThreads) {
+        const int row = fd_fw.div(i), x = i - row * f_w;
+        const int kk = fd_rh.div(row), y = row - kk * rh;
+        const uint8_t *src = reinterpret_cast<const uint8_t *>(xrow0 + kk * strip_w) + y * S_w + c0 + s_xw[x];
+        const float *w = s_ww + x * tw;
+        float acc = 0.f;
+        for (int t = 0; t < tw; ++t) acc = fmaf(w[t], (float)src[t], acc);
+        s_t1[i] = acc;
+    }
+}
+
+// Glimpse H pass over nfr frames of t1 (rh x f_w each): tile byte (k, y, x) = rint(sum_t w[y][t] * t1[k][xh[y] + t][x]),
+// fp32 in the tap order of resample_h.  Output index i is the tile's byte offset: words straddle rows at f_w = 30.
+__device__ __forceinline__ void glimpse_hpass(const float *s_t1, int rh, const int32_t *s_xh, const float *s_wh, int th,
+                                              uint8_t *tb, int f_h, int f_w, int nfr, int tid, const uint32_t *s_magic) {
+    const FastDiv fd_fw(f_w, s_magic), fd_fh(f_h, s_magic);
+    for (int i = tid; i < nfr * f_h * f_w; i += kFlexThreads) {
+        const int row = fd_fw.div(i), x = i - row * f_w;
+        const int kk = fd_fh.div(row), y = row - kk * f_h;
+        const float *src = s_t1 + (kk * rh + s_xh[y]) * f_w + x;
+        const float *w = s_wh + y * th;
+        float acc = 0.f;
+        for (int t = 0; t < th; ++t) acc = fmaf(w[t], src[t * f_w], acc);
+        tb[i] = (uint8_t)quant_u8(acc);
+    }
+}
+
 template <int VARIANT>
 __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(const __grid_constant__ DevPlan p,
                                                                           const uint8_t *__restrict__ ring,
@@ -386,7 +433,7 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
                                                                           const uint8_t *__restrict__ ctrl,
                                                                           int32_t *__restrict__ loc, int32_t *__restrict__ res,
                                                                           int oh, int ow, int t1_cap, uint8_t *__restrict__ out,
-                                                                          int *__restrict__ counters) {
+                                                                          int *__restrict__ counters, int word_store) {
     extern __shared__ __align__(16) uint8_t smem[];
     constexpr int kWin = 4;
     // per claimed env: index, window, ring head, and where its operators live in the pool
@@ -402,8 +449,8 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
     const int K = p.K, quads = p.S_w >> 2, xcap = quads + 2, strip_w = (p.plane + 16) >> 2;
     const int tile_bytes = K * oh * ow;
     uint32_t *s_tile = reinterpret_cast<uint32_t *>(smem);                          // [K][oh][ow] bytes
-    uint32_t *s_x = s_tile + (tile_bytes >> 2);                                     // [K][strip_w]: the windows' full-width row strips
-    float *s_t1 = reinterpret_cast<float *>(smem + align16((size_t)tile_bytes + 4 * (size_t)K * p.S_h * xcap));  // [kg * rh][rwp]
+    uint32_t *s_x = reinterpret_cast<uint32_t *>(smem + align16((size_t)tile_bytes));  // [K][strip_w]: the windows' full-width row strips
+    float *s_t1 = reinterpret_cast<float *>(smem + align16(align16((size_t)tile_bytes) + 4 * (size_t)K * p.S_h * xcap));  // [kg * rh][rwp]
     uint32_t *s_wq = reinterpret_cast<uint32_t *>(s_t1 + t1_cap);                   // [rw][halves][4]; t1_cap % 4 == 0
     uint64_t *s_wh2 = reinterpret_cast<uint64_t *>(s_wq + p.S_w * 8);               // [rh][th] {w, w}
     int32_t *s_xw = reinterpret_cast<int32_t *>(s_wh2 + p.S_h * p.blur_tmax);       // [rw] first tap
@@ -454,7 +501,11 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
         const int n = q.n;
         loc[2 * n] = r; loc[2 * n + 1] = c; res[2 * n] = rh; res[2 * n + 1] = rw;
         s_er[e] = r; s_ec[e] = c; s_erh[e] = rh; s_erw[e] = rw; s_ehd[e] = q.hd;
-        if (rh > p.f_h) {
+        if constexpr (VARIANT == AGYM_OUT_RESIZE_FOV) {   // r -> f on both axes (family 0)
+            const FlexEntry eh = p.flex[rh], ew = p.flex[3 * (p.S_max + 1) + rw];
+            s_eth[e] = eh.taps; s_ehw[e] = eh.w_off; s_ehx[e] = eh.xmin_off;
+            s_enh[e] = ew.taps; s_eqw[e] = ew.w_off; s_eqx[e] = ew.xmin_off;
+        } else if (rh > p.f_h) {
             const FlexEntry eh = p.flexh2[rh], ew = p.flexq[rw];
             s_eth[e] = eh.taps; s_ehw[e] = eh.w_off; s_ehx[e] = eh.xmin_off;
             s_enh[e] = ew.taps; s_eqw[e] = ew.w_off; s_eqx[e] = ew.xmin_off;
@@ -480,7 +531,13 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
     // ---- workers: the W operator of entry e by cp.async (one group)
     auto prefetch = [&](int e) {
         const int n = s_en[e];
-        if (n < N && s_erh[e] > p.f_h) {
+        if constexpr (VARIANT == AGYM_OUT_RESIZE_FOV) {   // f_w rows of fp32 weights (the pool is only 4-byte aligned)
+            if (n < N) {
+                const int32_t *gq = p.pool_i + s_eqw[e], *gx = p.pool_i + s_eqx[e];
+                for (int i = tid; i < p.f_w * s_enh[e]; i += kFlexThreads) cp_async4(s_wq + i, gq + i);
+                for (int i = tid; i < p.f_w; i += kFlexThreads) cp_async4(s_xw + i, gx + i);
+            }
+        } else if (n < N && s_erh[e] > p.f_h) {
             const int rw = s_erw[e];
             const int32_t *gq = p.pool_i + s_eqw[e], *gx = p.pool_i + s_eqx[e];
             for (int i = tid; i < rw * s_enh[e]; i += kFlexThreads) cp_async16(s_wq + 4 * i, gq + 4 * i);
@@ -520,7 +577,15 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
         g.m_last = word_mask(4 * (g.nq - 1), sb, sb + vw);
         const uint32_t *s_xs = s_x + ((r0 * p.S_w & 15) >> 2);   // first window row of frame 0 (behind the hull's lead)
         int th = 1, nh = 1;
-        if (blur) {  // this env's H operator; s_wh2 / s_xh were last read before the previous env's final barrier
+        if constexpr (VARIANT == AGYM_OUT_RESIZE_FOV) {   // this env's H operator (f_h rows), as below
+            th = s_eth[e];
+            nh = s_enh[e];
+            if (worker) {
+                const int32_t *gh = p.pool_i + s_ehw[e], *gx = p.pool_i + s_ehx[e];
+                for (int i = tid; i < p.f_h * th; i += kFlexThreads) cp_async4(reinterpret_cast<float *>(s_wh2) + i, gh + i);
+                for (int i = tid; i < p.f_h; i += kFlexThreads) cp_async4(s_xh + i, gx + i);
+            }
+        } else if (blur) {  // this env's H operator; s_wh2 / s_xh were last read before the previous env's final barrier
             th = s_eth[e];
             nh = s_enh[e];
             if (worker) {
@@ -540,17 +605,20 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
             if (n2 >= N) { n2 = N; more = false; }
             load_env(n2, pend);
         }
-        if (worker) {   // zero frame (everything outside the window stays zero)
+        if (worker && VARIANT != AGYM_OUT_RESIZE_FOV) {   // zero frame (everything outside the window stays zero)
             const uint4 z4 = make_uint4(0u, 0u, 0u, 0u);
             for (int i = tid; i < (tile_bytes >> 4); i += kFlexThreads) reinterpret_cast<uint4 *>(s_tile)[i] = z4;
         }
-        const int per = blur ? rh * g.rwp : rh * g.nq;
+        const int per = VARIANT == AGYM_OUT_RESIZE_FOV ? rh * ow : blur ? rh * g.rwp : rh * g.nq;
         const int kg = min(K, t1_cap / per);
         for (int k0 = 0; k0 < K; k0 += kg) {
             const int kc = min(kg, K - k0);
             const bool last = k0 + kc >= K;
             if (k0) __syncthreads();           // the previous group's H pass has read t1
             if (!worker) {
+            } else if (VARIANT == AGYM_OUT_RESIZE_FOV) {
+                glimpse_wpass(s_xs + k0 * strip_w, rh, p.S_w, strip_w, s_xw, reinterpret_cast<const float *>(s_wq), nh, s_t1, ow, c0,
+                              kc * rh, tid, s_magic);
             } else if (blur) {
                 if (nh == 1) flex_wpass<1>(s_xs + k0 * strip_w, rh, quads, strip_w, s_xw, s_wq, s_t1, g.rwp, sb, c0, rw, kc * rh, tid, s_magic);
                 else flex_wpass<2>(s_xs + k0 * strip_w, rh, quads, strip_w, s_xw, s_wq, s_t1, g.rwp, sb, c0, rw, kc * rh, tid, s_magic);
@@ -570,7 +638,7 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
                     t1w[i] = word;
                 }
             }
-            if (last) cp_async_wait<0>();      // H operator
+            if (last || VARIANT == AGYM_OUT_RESIZE_FOV) cp_async_wait<0>();      // H operator
             __syncthreads();                   // #2: t1 complete; after the last group s_x / s_wq / s_xw are free
             if (last && boss) {
                 fetch_strips((j + 1) & (kWin - 1));                    // s_x is free: the next env's windows
@@ -578,7 +646,10 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
             }
             if (!worker) continue;
             if (last) prefetch((j + 1) & (kWin - 1));
-            if (blur) {
+            if (VARIANT == AGYM_OUT_RESIZE_FOV) {
+                glimpse_hpass(s_t1, rh, s_xh, reinterpret_cast<const float *>(s_wh2), th, reinterpret_cast<uint8_t *>(s_tile) + k0 * oh * ow,
+                              oh, ow, kc, tid, s_magic);
+            } else if (blur) {
                 switch (th) {
                     case 3: flex_hpass<3>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
                     case 4: flex_hpass<4>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
@@ -598,15 +669,26 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
         }
         fence_async_smem();
         __syncthreads();                       // #3: tile complete
-        if (boss) {
+        const bool words = VARIANT == AGYM_OUT_RESIZE_FOV && word_store;
+        if (boss && !words) {
             bulk_s2g(out + (size_t)n * tile_bytes, s_tile, (uint32_t)tile_bytes);
             bulk_commit();
         }
-        if (p.norm_out) {   // uniform: the normalised copy of the finished tile; the tile is next written after barrier #1 of
-                            // the following env, which comes after this loop in every thread's program order
-            const uint4 *t4 = reinterpret_cast<const uint4 *>(s_tile);
-            const int nv = tile_bytes >> 4;
-            for (int i = threadIdx.x; i < nv; i += (int)blockDim.x) norm_store16(p.norm_dt, t4[i], p.norm_out, (size_t)n * nv + i);
+        // uniform: the tile leaves as words, or its normalised copy is written; the tile is next written after barrier #1
+        // of the following env, which comes after this in every thread's program order
+        if (words) {
+            uint32_t *o = reinterpret_cast<uint32_t *>(out + (size_t)n * tile_bytes);
+            for (int i = threadIdx.x; i < (tile_bytes >> 2); i += (int)blockDim.x) o[i] = s_tile[i];
+        }
+        if (p.norm_out) {
+            if (VARIANT == AGYM_OUT_RESIZE_FOV && (tile_bytes & 15)) {
+                const int nw = tile_bytes >> 2;
+                for (int i = threadIdx.x; i < nw; i += (int)blockDim.x) norm_store4(p.norm_dt, s_tile[i], p.norm_out, (size_t)n * nw + i);
+            } else {
+                const uint4 *t4 = reinterpret_cast<const uint4 *>(s_tile);
+                const int nv = tile_bytes >> 4;
+                for (int i = threadIdx.x; i < nv; i += (int)blockDim.x) norm_store16(p.norm_dt, t4[i], p.norm_out, (size_t)n * nv + i);
+            }
         }
     }
     cp_async_wait<0>();
@@ -627,19 +709,23 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
     DevPlan q = p;
     q.err = err;
     q.norm_out = norm_out; q.norm_dt = norm_dt;
-    const size_t out_bytes = (size_t)p.N * p.K * (variant == AGYM_OUT_CROP ? (size_t)pad_h * pad_w : (size_t)p.plane);
+    const size_t out_bytes = (size_t)p.N * p.K *
+                             (variant == AGYM_OUT_CROP ? (size_t)pad_h * pad_w : variant == AGYM_OUT_RESIZE_FOV ? (size_t)p.f_h * p.f_w : (size_t)p.plane);
     auto finish = [&](cudaError_t r) {   // kernels without the fused normalised store: a separate pass over the u8 output
         if (r != cudaSuccess || !norm_out) return r;
         if (out_bytes % 16 != 0) return cudaErrorInvalidValue;
         return launch_normalize(out, out_bytes, norm_dt, norm_out, st);
     };
+    const bool glimpse = variant == AGYM_OUT_RESIZE_FOV;
     if (variant != AGYM_OUT_RESIZE_FULL && p.flexb && p.flexq && !g_disable_std && !g_flex_old) {
         // persistent kernel, 2 CTAs per SM: whatever the fixed buffers leave of ~113 KB goes to t1
-        const int oh = variant == AGYM_OUT_CROP ? pad_h : p.S_h, ow = variant == AGYM_OUT_CROP ? pad_w : p.S_w;
+        const int oh = variant == AGYM_OUT_CROP ? pad_h : glimpse ? p.f_h : p.S_h;
+        const int ow = variant == AGYM_OUT_CROP ? pad_w : glimpse ? p.f_w : p.S_w;
         const size_t tile = (size_t)p.K * oh * ow;
-        const size_t fixed = a16(tile + 4 * (size_t)p.K * p.S_h * (p.S_w / 4 + 2)) +
+        const size_t fixed = a16(a16(tile) + 4 * (size_t)p.K * p.S_h * (p.S_w / 4 + 2)) +
                              4 * ((size_t)p.S_w * 8 + 2 * (size_t)p.S_h * p.blur_tmax + p.S_w + p.S_h) + 16;
-        const size_t one = (size_t)p.S_h * (p.S_w + 4), all = (size_t)p.K * one;   // floats: one / all K frames of the largest window
+        // floats: one / all K frames of the largest window (the glimpse keeps f_w columns of each window row)
+        const size_t one = (size_t)p.S_h * (glimpse ? p.f_w : p.S_w + 4), all = (size_t)p.K * one;
         // + static shared memory + 1 KB reserved per CTA: two CTAs per SM (233,472 B).  RGB plans whose fixed buffers do
         // not leave one window's t1 in that budget (mask_out at 3 frames x 3 planes: 133 KB of tile and strips) run
         // one CTA per SM with the whole SM's shared memory instead
@@ -647,9 +733,15 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
         const size_t budget = ctas_per_sm == 2 ? 114000 : 225000;
         const size_t room = budget > fixed ? ((budget - fixed) / 4) & ~size_t(3) : 0;
         const size_t t1_cap = std::min(all, room);
-        if (tile % 16 == 0 && ow % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && t1_cap >= one &&
-            p.plane % 16 == 0 && p.S_w % 4 == 0 && (reinterpret_cast<uintptr_t>(ring) & 15) == 0 &&   // strip copies
-            (size_t)p.K * p.f_h * (p.S_w / 4 + 1) <= t1_cap) {
+        // the glimpse's tile leaves by the bulk store when it can, as 4-byte words otherwise; its fp32 operators take the
+        // places of the fixed-point W operator (S_w * 8 words) and the duplicated H operator (2 * S_h * blur_tmax words)
+        const bool bulk_out = tile % 16 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0;
+        const bool out_ok = glimpse ? tile % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 3) == 0 &&
+                                          (size_t)p.f_w * p.fov_tmax <= (size_t)p.S_w * 8 &&
+                                          (size_t)p.f_h * p.fov_tmax <= 2 * (size_t)p.S_h * p.blur_tmax
+                                    : bulk_out && ow % 4 == 0 && (size_t)p.K * p.f_h * (p.S_w / 4 + 1) <= t1_cap;
+        if (out_ok && t1_cap >= one &&
+            p.plane % 16 == 0 && p.S_w % 4 == 0 && (reinterpret_cast<uintptr_t>(ring) & 15) == 0) {   // strip copies
             const size_t fs = fixed + 4 * t1_cap;
             int dev = 0, sms = 148;
             cudaGetDevice(&dev);
@@ -659,15 +751,18 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
             if ((e = cudaMemsetAsync(p.flex_counters, 0, 16, st)) != cudaSuccess) return e;
             if (variant == AGYM_OUT_CROP) {
                 if ((e = set_smem(k_observe_flexible_v3<AGYM_OUT_CROP>, fs)) != cudaSuccess) return e;
-                k_observe_flexible_v3<AGYM_OUT_CROP><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters);
+                k_observe_flexible_v3<AGYM_OUT_CROP><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, 0);
+            } else if (glimpse) {
+                if ((e = set_smem(k_observe_flexible_v3<AGYM_OUT_RESIZE_FOV>, fs)) != cudaSuccess) return e;
+                k_observe_flexible_v3<AGYM_OUT_RESIZE_FOV><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, bulk_out ? 0 : 1);
             } else {
                 if ((e = set_smem(k_observe_flexible_v3<AGYM_OUT_MASK>, fs)) != cudaSuccess) return e;
-                k_observe_flexible_v3<AGYM_OUT_MASK><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters);
+                k_observe_flexible_v3<AGYM_OUT_MASK><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, 0);
             }
             return cudaGetLastError();
         }
     }
-    if (variant != AGYM_OUT_RESIZE_FULL && p.flexb && !g_disable_std) {
+    if ((variant == AGYM_OUT_CROP || variant == AGYM_OUT_MASK) && p.flexb && !g_disable_std) {
         const int oh = variant == AGYM_OUT_CROP ? pad_h : p.S_h, ow = variant == AGYM_OUT_CROP ? pad_w : p.S_w;
         const size_t tile = (size_t)p.K * oh * ow;
         // t1: one padded window of any size (S_h x S_w), or all K frames of windows up to ~50 x 52
@@ -691,6 +786,7 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
     k_observe_flexible<V><<<p.N, kThreads, smem, st>>>(q, ring, head, action, atype, ctrl, loc, res, pad_h, pad_w, out);
     if (variant == AGYM_OUT_CROP) { AGYM_LAUNCH_FLEX(AGYM_OUT_CROP) }
     else if (variant == AGYM_OUT_MASK) { AGYM_LAUNCH_FLEX(AGYM_OUT_MASK) }
+    else if (glimpse) { AGYM_LAUNCH_FLEX(AGYM_OUT_RESIZE_FOV) }
     else { AGYM_LAUNCH_FLEX(AGYM_OUT_RESIZE_FULL) }
 #undef AGYM_LAUNCH_FLEX
     return finish(cudaGetLastError());

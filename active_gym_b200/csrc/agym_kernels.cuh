@@ -36,6 +36,7 @@ struct DevPlan {
     AxisRef full_w, full_h; // resize_to_full f -> S (fov_env.py:120,182)
     // flexible fovea tables: index [axis][family][r], family 0 = r->f, 1 = f->r, 2 = r->S
     const FlexEntry *flex;  // [2][3][S_max+1]
+    int32_t fov_tmax;       // widest r->f table (family 0) over both axes and every r
     // composed blur (Resize(f) then Resize(r)) per axis and window size r: [2][S_max+1]; blur_tmax = widest band
     const FlexEntry *flexb;
     int32_t blur_tmax;

@@ -23,7 +23,7 @@ from .spaces import Box
 
 
 class DMCEnvArgs:
-    """Source-compatible with dmc_env.py:56-76 (+ ``resize_to_full`` default, see AtariEnvArgs)."""
+    """Source-compatible with dmc_env.py:56-76 (+ ``resize_to_full`` and ``resize_to_fov`` defaults, see AtariEnvArgs)."""
 
     def __init__(self, domain_name: str, task_name: str, seed: int, obs_size: Tuple[int, int], **kwargs):
         self.env_backend = "dmc"
@@ -43,6 +43,7 @@ class DMCEnvArgs:
         self.clip_reward = False
         self.record = False
         self.resize_to_full = False
+        self.resize_to_fov = False
         for k, v in kwargs.items():
             self.__setattr__(k, v)
 

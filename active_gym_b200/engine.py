@@ -21,7 +21,8 @@ from . import _lib
 LUMA_RGB = (9798, 19235, 3735)
 LUMA_DMC = (3735, 19235, 9798)
 
-VARIANTS = {"crop": _lib.OUT_CROP, "mask": _lib.OUT_MASK, "resize_full": _lib.OUT_RESIZE_FULL}
+VARIANTS = {"crop": _lib.OUT_CROP, "mask": _lib.OUT_MASK, "resize_full": _lib.OUT_RESIZE_FULL,
+            "resize_fov": _lib.OUT_RESIZE_FOV}
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -215,6 +216,8 @@ class ObservationPath:
         NK, S = (self.n_envs,) + self._frame_axes(), self.obs_size
         if kind == "peripheral" or variant in ("mask", "resize_full"):
             return NK + S
+        if kind == "flexible" and variant == "resize_fov":   # the glimpse: every window resampled to fov_size
+            return NK + self.fov_size
         if kind == "flexible":
             return NK + tuple(pad if pad is not None else S)
         return NK + self.fov_size

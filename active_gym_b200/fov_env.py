@@ -334,11 +334,19 @@ class FlexibleFovealEnvActionType(IntEnum):  # fov_env.py:236-238
 class FlexibleFovealEnv(FixedFovealEnv):
     """fov_env.py:240-355 for N envs.  Without mask_out / resize_to_full the reference returns a
     variable-shape (K, rh, rw) crop; the batched form writes it into the top-left corner of a
-    zeroed (N, K, S_h, S_w) tensor and reports the shape in ``info["fov_res"]``."""
+    zeroed (N, K, S_h, S_w) tensor and reports the shape in ``info["fov_res"]``.
+
+    ``args.resize_to_fov`` (superset, default False): the observation is the glimpse, a fixed-shape (N, K, f_h, f_w)
+    tensor — each plane's unblurred window after this step's fovea update, resampled to fov_size by torchvision's
+    ``Resize(fov_size)`` (fov_env.py:248,284-285) under the same ``antialias`` switch.  It excludes ``mask_out`` and
+    ``resize_to_full``."""
 
     _kind = "flexible"
 
     def __init__(self, env, args):
+        self.resize_to_fov = bool(getattr(args, "resize_to_fov", False))
+        if self.resize_to_fov and (bool(getattr(args, "mask_out", False)) or bool(getattr(args, "resize_to_full", False))):
+            raise ValueError("resize_to_fov excludes mask_out and resize_to_full: each selects a different observation")
         super().__init__(env, args)
         self.action_space["sensory_action_type"] = Discrete(len(FlexibleFovealEnvActionType))
         self.fov_init_res = tuple(args.fov_size)
@@ -347,6 +355,10 @@ class FlexibleFovealEnv(FixedFovealEnv):
     @property
     def fov_res(self) -> torch.Tensor:
         return self.path.res
+
+    @property
+    def variant(self) -> str:
+        return "resize_fov" if self.resize_to_fov else super().variant
 
     def _check_res(self, action, action_type):
         """The reference raises for a window larger than the frame; do it before the launch

@@ -79,6 +79,9 @@ typedef enum agym_status {
 #define AGYM_OUT_CROP 0          /* (K, f_h, f_w); flexible: padded (K, pad_h, pad_w)         */
 #define AGYM_OUT_MASK 1          /* mask_out: (K, S_h, S_w), zero outside the fovea           */
 #define AGYM_OUT_RESIZE_FULL 2   /* resize_to_full: (K, S_h, S_w)                             */
+#define AGYM_OUT_RESIZE_FOV 3    /* flexible only: resize_to_fov, (K, f_h, f_w) = Resize(fov_size) of the unblurred window.
+                                    Added without an ABI version bump (the struct and every signature are unchanged):
+                                    a library that predates it rejects variant 3 with AGYM_ERR_INVALID_ARG */
 
 /* bits of the device error word of agym_observe_flexible (d_err): FOV_RES actions the reference would fail on
  * (fov_env.py:322-324 stores the action unvalidated; the crop then raises for float bounds or a window larger than
@@ -183,6 +186,11 @@ AGYM_API int agym_observe_peripheral(const agym_plan *plan, const uint8_t *d_rin
 /* Replaces FlexibleFovealEnv._fov_step + _get_fov_state (fov_env.py:270-330).
  * d_atype: i32 [N] (NULL = all FOV_LOC).  CROP writes the variable-size patch into the
  * top-left corner of a zeroed [N][K][pad_h][pad_w] buffer (pad >= the largest res).
+ * RESIZE_FOV writes the glimpse u8 [N][K][f_h][f_w]: each plane's unblurred window after this call's fovea update,
+ * resampled to fov_size (torchvision Resize(fov_size), fov_env.py:248,284-285; the first half of the reference's blur),
+ * within 0.5 LSB + 0.01 of the reference's float value (fp32 weights and accumulation on both axes); pad_h / pad_w are
+ * ignored.  Any d_out alignment and any fov_size are served: the fast kernel when the tile K*f_h*f_w is a multiple of
+ * 4 bytes and d_out is 4-byte aligned, the table-driven kernel otherwise.
  * Blurred pixels (res rows > fov rows) are within 0.5 LSB + 0.02 of the reference's float value: the W-axis
  * operator runs in 16-bit fixed point (<= 255 * taps / 2^17 LSB from the fp64 weights); windows that the
  * reference does not blur, the mask and the padding are bit exact.

@@ -10,14 +10,16 @@ from .engine import LUMA_DMC, LUMA_RGB, ObservationPath  # noqa: F401
 from .pipeline import PipelinedPath  # noqa: F401
 from .vector import FovealVectorEnv, ShardedVecEnv  # noqa: F401
 from .atari_env import (  # noqa: F401
-    AtariBaseEnv, AtariEnvArgs, AtariFixedFovealEnv, AtariFixedFovealPeripheralEnv, AtariFlexibleFovealEnv, AtariVecEnv,
+    AtariBaseEnv, AtariEnvArgs, AtariFixedFovealEnv, AtariFixedFovealPeripheralEnv, AtariFlexibleFovealEnv,
+    AtariFlexibleFovealPeripheralEnv, AtariVecEnv,
 )
 from .dmc_env import (  # noqa: F401
-    DMCBaseEnv, DMCEnvArgs, DMCFixedFovealEnv, DMCFixedFovealPeripheralEnv, DMCFlexibleFovealEnv, DMCVecEnv,
+    DMCBaseEnv, DMCEnvArgs, DMCFixedFovealEnv, DMCFixedFovealPeripheralEnv, DMCFlexibleFovealEnv,
+    DMCFlexibleFovealPeripheralEnv, DMCVecEnv,
 )
 from .fov_env import (  # noqa: F401
-    FixedFovealEnv, FixedFovealPeripheralEnv, FlexibleFovealEnv, FlexibleFovealEnvActionType, RecordWrapper,
-    SingleEnvAdapter,
+    FixedFovealEnv, FixedFovealPeripheralEnv, FlexibleFovealEnv, FlexibleFovealEnvActionType,
+    FlexibleFovealPeripheralEnv, RecordWrapper, SingleEnvAdapter,
 )
 
 __all__ = [
@@ -26,4 +28,6 @@ __all__ = [
     "RecordWrapper", "FixedFovealEnv", "FlexibleFovealEnv", "FlexibleFovealEnvActionType", "FixedFovealPeripheralEnv",
     "AtariVecEnv", "DMCVecEnv", "SingleEnvAdapter", "ObservationPath", "PipelinedPath", "FovealVectorEnv", "ShardedVecEnv",
     "LUMA_RGB", "LUMA_DMC",
+    # supersets of the reference
+    "AtariFlexibleFovealPeripheralEnv", "DMCFlexibleFovealPeripheralEnv", "FlexibleFovealPeripheralEnv",
 ]

@@ -29,6 +29,7 @@ EXPORTS = (
     "agym_plan_ring_bytes", "agym_plan_pcache_bytes", "agym_ingest_atari", "agym_ingest_dmc",
     "agym_stack", "agym_observe_fixed", "agym_observe_peripheral", "agym_observe_flexible",
     "agym_synth_frames", "agym_table_cv2", "agym_table_aa", "agym_table_blur", "agym_normalize", "agym_plan_used_rows", "agym_ingest_atari_packed", "agym_record_step",
+    "agym_observe_flexible_peripheral",
 )
 
 
@@ -73,6 +74,7 @@ def lib() -> C.CDLL:
     L.agym_observe_fixed.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, vp, i32, vp]
     L.agym_observe_peripheral.argtypes = [vp] * 9 + [i32, vp]
     L.agym_observe_flexible.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, i32, vp]
+    L.agym_observe_flexible_peripheral.argtypes = [vp] * 12 + [i32, vp]
     L.agym_record_step.argtypes = [i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.agym_synth_frames.argtypes = [vp, sz, u64, vp]
     L.agym_normalize.argtypes = [vp, sz, i32, vp, vp]

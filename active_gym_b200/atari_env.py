@@ -231,3 +231,10 @@ def AtariFixedFovealPeripheralEnv(args, num_envs: Optional[int] = None, source=N
     from .fov_env import FixedFovealPeripheralEnv, SingleEnvAdapter
     env = FixedFovealPeripheralEnv(AtariBaseEnv(args, num_envs or 1, source, device), args)
     return SingleEnvAdapter(env) if num_envs is None else env
+
+
+def AtariFlexibleFovealPeripheralEnv(args, num_envs: Optional[int] = None, source=None, device=None):
+    """Superset: the flexible fovea over the peripheral background (fov_env.FlexibleFovealPeripheralEnv)."""
+    from .fov_env import FlexibleFovealPeripheralEnv, SingleEnvAdapter
+    env = FlexibleFovealPeripheralEnv(AtariBaseEnv(args, num_envs or 1, source, device), args)
+    return SingleEnvAdapter(env) if num_envs is None else env

@@ -543,8 +543,20 @@ int agym_observe_flexible(const agym_plan *plan, const uint8_t *d_ring, const in
                           : variant == AGYM_OUT_RESIZE_FOV ? static_cast<size_t>(c.fov_h) * c.fov_w
                                                            : static_cast<size_t>(c.obs_h) * c.obs_w);
     if ((v = check_norm_args(d_out, bytes, d_out_norm, norm_dtype)) != AGYM_OK) return v;
-    return ret(launch_observe_flexible(plan->dev, d_ring, d_head, d_action, d_atype, d_fov_ctrl, d_loc, d_res, variant,
+    return ret(launch_observe_flexible(plan->dev, d_ring, d_head, nullptr, d_action, d_atype, d_fov_ctrl, d_loc, d_res, variant,
                                        pad_h, pad_w, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));
+}
+
+int agym_observe_flexible_peripheral(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head, const float *d_pcache,
+                                     const double *d_action, const int32_t *d_atype, const uint8_t *d_fov_ctrl, int32_t *d_loc,
+                                     int32_t *d_res, uint8_t *d_out, int32_t *d_err, void *d_out_norm, int norm_dtype, void *stream) {
+    int v = check_fov_args(plan, d_ring, d_head, d_action, d_fov_ctrl, d_loc, d_out);
+    if (v != AGYM_OK) return v;
+    if (plan->cfg.periph_h == 0 || !d_pcache || !d_res) return AGYM_ERR_INVALID_ARG;
+    const agym_config &c = plan->cfg;
+    if ((v = check_norm_args(d_out, static_cast<size_t>(c.n_envs) * ring_planes(c) * c.obs_h * c.obs_w, d_out_norm, norm_dtype)) != AGYM_OK) return v;
+    return ret(launch_observe_flexible(plan->dev, d_ring, d_head, d_pcache, d_action, d_atype, d_fov_ctrl, d_loc, d_res, kOutPeriph,
+                                       0, 0, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));
 }
 
 int agym_table_cv2(int n_src, int n_dst, int zero_frac_at_border, int32_t *h_s0, int32_t *h_s1, int32_t *h_coef) {

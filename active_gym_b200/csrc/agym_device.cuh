@@ -202,6 +202,12 @@ __device__ __forceinline__ uint4 luma16(const uint32_t (&w)[12], uint32_t w01, u
 
 __device__ __forceinline__ size_t align16(size_t v) { return (v + 15) & ~size_t(15); }
 
+// Two-tap expand of the cached squeeze (the peripheral kernels and the flexible fovea's peripheral background): lerp
+// weights sum to one, so a bias of 49152.5 added in the W pass rides through both passes and the rounded pixel
+// floor(v + 0.5) ends up in byte 1 of the float's bit pattern (ulp there is 2^-8, so the total evaluation error is
+// < 0.01 u8 LSB) — no float->int conversion, one PRMT tree per 4 pixels.
+constexpr float kBias = 49152.5f;
+
 // Squeeze of one obs frame held in shared memory (u8) into the peripheral cache slot:
 // Resize(peripheral_res) = W pass then H pass (fov_env.py:367).  Needs t1[S_h * p_w] floats.
 __device__ void squeeze_to_cache(const DevPlan &p, const uint8_t *s_frame, float *s_t1, float *dst_global, int tid, int nt) {

@@ -16,6 +16,109 @@ __device__ __forceinline__ AxisRef flex_axis(const DevPlan &p, int axis, int fam
     return a;
 }
 
+// Peripheral background of the flexible fovea, Resize(obs_size) of the cached squeeze (fov_env.py:366-368, 376): rows
+// [y0, y1) of column quad q of one plane, from that plane's squeeze sq [p_h][p_w] and the plan's two-tap expand tables.
+// The arithmetic is k_observe_peripheral_std's: W pass T = fma(w1, s[i0 + 1], fma(w0, s[i0], kBias)), H pass
+// fma(w0, T[j] - T[j + 1], T[j + 1]), the pixel in byte 1 of the float; so the background is bit-identical to that
+// kernel's at the standard geometry (its clamped border rows read T[0] twice: T[0] - T[1] and T[1] + (T[0] - T[1]) are
+// exact, all T lying in [2^15, 2^16)).  dst: the word of row y0; rows are dstride words apart.
+__device__ __forceinline__ void periph_expand(const DevPlan &p, const float *sq, int q, int y0, int y1, uint32_t *dst,
+                                              int dstride) {
+    int i0[4];
+    float w0[4], w1[4], a[4], b[4];
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+        i0[c] = __ldg(p.exw_i0 + 4 * q + c);
+        w0[c] = __ldg(p.exw_w0 + 4 * q + c);
+        w1[c] = __ldg(p.exw_w1 + 4 * q + c);
+    }
+    int j_have = -2;
+    for (int y = y0; y < y1; ++y, dst += dstride) {
+        const int j = __ldg(p.exh_i0 + y);
+        const float wh = __ldg(p.exh_w0 + y);
+        if (j != j_have) {   // squeezed rows j, j + 1 W-expanded (row j is the previous row j + 1 when the pair moves by one)
+            const float *sa = sq + j * p.p_w, *sb = sa + p.p_w;
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+                a[c] = j == j_have + 1 ? b[c] : fmaf(w1[c], sa[i0[c] + 1], fmaf(w0[c], sa[i0[c]], kBias));
+                b[c] = fmaf(w1[c], sb[i0[c] + 1], fmaf(w0[c], sb[i0[c]], kBias));
+            }
+            j_have = j;
+        }
+        uint32_t word = 0u;
+#pragma unroll
+        for (int c = 0; c < 4; ++c) word |= ((__float_as_uint(fmaf(wh, a[c] - b[c], b[c])) >> 8) & 0xffu) << (8 * c);
+        *dst = word;
+    }
+}
+
+// One plane of the table-driven kernel's peripheral variant: the window (bufA, rh x rw floats of its bytes), blurred iff
+// rh > f_h in the arithmetic of the kernel that serves agym_observe_flexible(AGYM_OUT_MASK) on the same plan — the
+// persistent kernel's 16-bit fixed-point W pass and fp32 H pass when the plan has those operators, the composed fp32
+// operators of k_observe_flexible_fast otherwise — pasted onto the background of periph_expand (or, for expand tables
+// that are not two-tap lerps, of k_observe_peripheral's generic passes).  Written byte by byte: out may sit at any address.
+__device__ void periph_plane(const DevPlan &p, float *bufA, float *bufB, uint32_t *s_bg, const float *sq, int r0, int c0,
+                             int rh, int rw, bool blur, uint8_t *out, int tid) {
+    const FastDiv fd_rw(rw);
+    if (blur) {
+        const bool fixed_w = p.flexq != nullptr;
+        const FlexEntry ew = fixed_w ? p.flexq[rw] : p.flexb[(p.S_max + 1) + rw];
+        const FlexEntry eh = fixed_w ? p.flexh2[rh] : p.flexb[rh];
+        for (int i = tid; i < rh * rw; i += kThreads) {   // W pass
+            const int y = fd_rw.div(i), x = i - y * rw;
+            const float *src = bufA + y * rw + __ldg(p.pool_i + ew.xmin_off + x);
+            if (fixed_w) {   // flexq: {xmin, q16 weights in halves of 8 taps, halves, taps}
+                const uint32_t *qw = reinterpret_cast<const uint32_t *>(p.pool_i + ew.w_off) + x * ew.taps * 4;
+                uint32_t acc = 0u;
+                for (int t = 0; t < ew.n_out; ++t) acc += ((__ldg(qw + (t >> 1)) >> (16 * (t & 1))) & 0xffffu) * (uint32_t)src[t];
+                bufB[i] = (float)acc * (1.f / 65536.f);
+            } else {
+                const float *w = reinterpret_cast<const float *>(p.pool_i + ew.w_off) + x * ew.taps;
+                float acc = 0.f;
+                for (int t = 0; t < ew.taps; ++t) acc = fmaf(__ldg(w + t), src[t], acc);
+                bufB[i] = acc;
+            }
+        }
+        __syncthreads();
+        const int wstep = fixed_w ? 2 : 1;   // flexh2 stores every weight twice
+        for (int i = tid; i < rh * rw; i += kThreads) {   // H pass
+            const int y = fd_rw.div(i), x = i - y * rw;
+            const float *src = bufB + __ldg(p.pool_i + eh.xmin_off + y) * rw + x;
+            const float *w = reinterpret_cast<const float *>(p.pool_i + eh.w_off) + wstep * y * eh.taps;
+            float acc = 0.f;
+            for (int t = 0; t < eh.taps; ++t) acc = fmaf(src[t * rw], __ldg(w + wstep * t), acc);
+            bufA[i] = acc;
+        }
+    }
+    const int quads = p.S_w >> 2;
+    if (p.fast_expand) {
+        const int nseg = min(p.S_h, max(1, kThreads / quads)), rows = (p.S_h + nseg - 1) / nseg;
+        for (int i = tid; i < quads * nseg; i += kThreads) {
+            const int g = i / quads, q = i - g * quads;
+            periph_expand(p, sq, q, g * rows, min(p.S_h, g * rows + rows), s_bg + g * rows * quads + q, quads);
+        }
+    } else {   // squeeze -> s_sq, W pass -> s_t2, H pass per word (k_observe_peripheral<true>)
+        float *s_sq = reinterpret_cast<float *>(s_bg + quads * p.S_h), *s_t2 = s_sq + p.p_h * p.p_w;
+        for (int i = tid; i < p.p_h * p.p_w; i += kThreads) s_sq[i] = __ldg(sq + i);
+        __syncthreads();
+        resample_w<float>(s_sq, p.p_w, s_t2, p.S_w, p.p_h, p.ex_w, tid, kThreads);
+        __syncthreads();
+        for (int t = tid; t < quads * p.S_h; t += kThreads) {
+            const int y = t / quads;
+            s_bg[t] = resample_h_word(s_t2, p.S_w, p.ex_h, y, 4 * (t - y * quads));
+        }
+    }
+    __syncthreads();
+    const uint8_t *bg = reinterpret_cast<const uint8_t *>(s_bg);
+    const FastDiv fd_sw(p.S_w);
+    for (int i = tid; i < p.plane; i += kThreads) {   // fov_env.py:385-386 at the flexible window
+        const int y = fd_sw.div(i), x = i - y * p.S_w;
+        const int py = y - r0, px = x - c0;
+        out[i] = (py >= 0 && py < rh && px >= 0 && px < rw) ? (uint8_t)quant_u8(bufA[py * rw + px]) : bg[i];
+    }
+    __syncthreads();
+}
+
 template <int VARIANT>
 __global__ void __launch_bounds__(kThreads) k_observe_flexible(const __grid_constant__ DevPlan p,
                                                                const uint8_t *__restrict__ ring,
@@ -24,7 +127,8 @@ __global__ void __launch_bounds__(kThreads) k_observe_flexible(const __grid_cons
                                                                const int32_t *__restrict__ atype,
                                                                const uint8_t *__restrict__ ctrl,
                                                                int32_t *__restrict__ loc, int32_t *__restrict__ res,
-                                                               int pad_h, int pad_w, uint8_t *__restrict__ out) {
+                                                               int pad_h, int pad_w, uint8_t *__restrict__ out,
+                                                               const float *__restrict__ pcache) {
     extern __shared__ __align__(16) uint8_t smem[];
     __shared__ int s_win[4];
     const int n = blockIdx.x, tid = threadIdx.x;
@@ -73,6 +177,12 @@ __global__ void __launch_bounds__(kThreads) k_observe_flexible(const __grid_cons
             bufA[i] = (float)__ldg(src + (r0 + y) * p.S_w + c0 + x);
         }
         __syncthreads();
+        if constexpr (VARIANT == kOutPeriph) {
+            periph_plane(p, bufA, bufB, reinterpret_cast<uint32_t *>(bufB + p.plane),
+                         pcache + ((size_t)n * p.K + (h + 1 + k) % p.K) * p.p_h * p.p_w, r0, c0, rh, rw, blur,
+                         out + ((size_t)n * p.K + k) * p.plane, tid);
+            continue;
+        }
         if (blur && VARIANT != AGYM_OUT_RESIZE_FOV) {  // Resize(fov_size) then Resize(fov_res) (fov_env.py:276-280)
             resample_w<float>(bufA, rw, bufB, p.f_w, rh, flex_axis(p, 1, 0, rw, rw), tid, kThreads);
             __syncthreads();
@@ -288,6 +398,10 @@ __global__ void __launch_bounds__(kThreads) k_observe_flexible_fast(const __grid
 // are fp32 with the r -> f tables of family 0, evaluated in the order of the table-driven kernel (bit-identical to it).
 // The tile is K * f_h * f_w bytes with no zero fill; a tile that is not a multiple of 16 bytes (f_w = 30 at K = 3 or
 // K * C = 9) or a 16-byte-misaligned output leaves as 4-byte words from the worker threads instead of the bulk store.
+// VARIANT kOutPeriph (agym_observe_flexible_peripheral) is mask_out over the peripheral background: the env's K-plane
+// squeeze (contiguous in pcache) arrives with the strips on the same mbarrier, the workers expand it into the tile where
+// mask_out zero-fills (periph_expand), and both paste paths merge the first / last word of every window row into that
+// background (FlexGeom::m_first / m_last) instead of overwriting its bytes with zeros.
 #ifndef AGYM_FLEX_THREADS
 #define AGYM_FLEX_THREADS 256
 #endif
@@ -299,10 +413,10 @@ struct FlexGeom {
     uint32_t m_first, m_last;  // byte masks of the first / last output word of a window row
 };
 
-// H pass over kc frames.  A thread OWNS an output word (window row y, word q): the row's weights, its first source row
+// H pass over kc frames (MERGE: over a background instead of zeros).  A thread OWNS an output word (window row y, word q): the row's weights, its first source row
 // and the word's byte mask stay in registers while the thread walks through the kc frames (pointer increments only) —
 // 25 instead of 70 instructions per output word for a 5-tap row.  s_wh2 holds every weight twice (FFMA2 operand).
-template <int TH>
+template <int TH, bool MERGE>
 __device__ __forceinline__ void flex_hpass(const FlexGeom &g, const float *s_t1, const uint64_t *s_wh2, const int32_t *s_xh,
                                            uint32_t *s_tile, int k0, int kc, int th, int tid, const uint32_t *s_magic) {
     const FastDiv fd_nq(g.nq, s_magic);
@@ -342,7 +456,8 @@ __device__ __forceinline__ void flex_hpass(const FlexGeom &g, const float *s_t1,
             uint32_t b0, b1, b2, b3;
             unpack2(fadd2(a01, rne2), b0, b1);
             unpack2(fadd2(a23, rne2), b2, b3);
-            *dst = __byte_perm(__byte_perm(b0, b1, 0x0040), __byte_perm(b2, b3, 0x0040), 0x5410) & mask;
+            const uint32_t v = __byte_perm(__byte_perm(b0, b1, 0x0040), __byte_perm(b2, b3, 0x0040), 0x5410) & mask;
+            *dst = MERGE ? (*dst & ~mask) | v : v;   // MERGE: the edge words keep the background's bytes
         }
     }
 }
@@ -433,9 +548,11 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
                                                                           const uint8_t *__restrict__ ctrl,
                                                                           int32_t *__restrict__ loc, int32_t *__restrict__ res,
                                                                           int oh, int ow, int t1_cap, uint8_t *__restrict__ out,
-                                                                          int *__restrict__ counters, int word_store) {
+                                                                          int *__restrict__ counters, int word_store,
+                                                                          const float *__restrict__ pcache) {
     extern __shared__ __align__(16) uint8_t smem[];
     constexpr int kWin = 4;
+    constexpr bool kPeriph = VARIANT == kOutPeriph;   // the window pasted onto the peripheral background
     // per claimed env: index, window, ring head, and where its operators live in the pool
     __shared__ int s_en[kWin], s_er[kWin], s_ec[kWin], s_erh[kWin], s_erw[kWin], s_ehd[kWin];
     __shared__ int s_eth[kWin], s_ehw[kWin], s_ehx[kWin], s_enh[kWin], s_eqw[kWin], s_eqx[kWin];
@@ -450,7 +567,10 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
     const int tile_bytes = K * oh * ow;
     uint32_t *s_tile = reinterpret_cast<uint32_t *>(smem);                          // [K][oh][ow] bytes
     uint32_t *s_x = reinterpret_cast<uint32_t *>(smem + align16((size_t)tile_bytes));  // [K][strip_w]: the windows' full-width row strips
-    float *s_t1 = reinterpret_cast<float *>(smem + align16(align16((size_t)tile_bytes) + 4 * (size_t)K * p.S_h * xcap));  // [kg * rh][rwp]
+    const int pp = p.p_h * p.p_w, sq_bytes = kPeriph ? 4 * K * pp : 0;
+    const size_t o_sq = align16(align16((size_t)tile_bytes) + 4 * (size_t)K * p.S_h * xcap);
+    float *s_sq = reinterpret_cast<float *>(smem + o_sq);                          // kPeriph: [K slots][p_h][p_w] squeeze
+    float *s_t1 = reinterpret_cast<float *>(smem + align16(o_sq + sq_bytes));     // [kg * rh][rwp]
     uint32_t *s_wq = reinterpret_cast<uint32_t *>(s_t1 + t1_cap);                   // [rw][halves][4]; t1_cap % 4 == 0
     uint64_t *s_wh2 = reinterpret_cast<uint64_t *>(s_wq + p.S_w * 8);               // [rh][th] {w, w}
     int32_t *s_xw = reinterpret_cast<int32_t *>(s_wh2 + p.S_h * p.blur_tmax);       // [rw] first tap
@@ -521,7 +641,8 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
         const uint32_t first = (uint32_t)(r0 * p.S_w), lead = first & 15u;
         const uint32_t bytes = (lead + (uint32_t)(rh * p.S_w) + 15u) & ~15u;
         const uint8_t *src = ring + (size_t)n * K * p.plane + (first - lead);
-        mbar_expect_tx(&s_bar, bytes * (uint32_t)K);
+        mbar_expect_tx(&s_bar, bytes * (uint32_t)K + (uint32_t)sq_bytes);
+        if (kPeriph) bulk_g2s(s_sq, pcache + (size_t)n * K * pp, (uint32_t)sq_bytes, &s_bar);   // the env's K slots, contiguous
         for (int k = 0; k < K; ++k) {
             int slot = h + 1 + k;
             slot -= slot >= K ? K : 0;
@@ -546,6 +667,16 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
         cp_async_commit();
     };
 
+    // kPeriph: background items (frame, row segment, column quad), nseg segments of `rows` rows per plane, chosen for
+    // the fewest rows per worker thread (3 x 28 rows at K = 4, 4 x 21 at K = 3 and K * C = 9)
+    int nseg = 1, rows = p.S_h;
+    if (kPeriph) {
+        for (int sg = 1, best = 1 << 30; sg <= 8; ++sg) {
+            const int cost = ((K * quads * sg + kFlexThreads - 1) / kFlexThreads) * ((p.S_h + sg - 1) / sg);
+            if (cost < best) { best = cost; nseg = sg; }
+        }
+        rows = (p.S_h + nseg - 1) / nseg;
+    }
     if (boss) {
         Pend q0, q1;
         load_env(min((int)blockIdx.x, N), q0);
@@ -565,7 +696,7 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
         if (boss) n2 = claim();                  // the env two iterations ahead; the result is not needed before #1
         const int r0 = s_er[e], c0 = s_ec[e], rh = s_erh[e], rw = s_erw[e];
         const bool blur = rh > p.f_h;  // row dimension only (fov_env.py:286)
-        const int oy = VARIANT == AGYM_OUT_MASK ? r0 : 0, ox = VARIANT == AGYM_OUT_MASK ? c0 : 0;
+        const int oy = VARIANT == AGYM_OUT_MASK || kPeriph ? r0 : 0, ox = VARIANT == AGYM_OUT_MASK || kPeriph ? c0 : 0;
         const int cb = c0 & 3, sb = ox & 3;
         const int vw = min(rw, ow - ox);
         FlexGeom g;
@@ -605,7 +736,16 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
             if (n2 >= N) { n2 = N; more = false; }
             load_env(n2, pend);
         }
-        if (worker && VARIANT != AGYM_OUT_RESIZE_FOV) {   // zero frame (everything outside the window stays zero)
+        if (worker && kPeriph) {   // the background: every plane expanded from its squeeze (s_sq is refilled after #2)
+            const FastDiv fd_q(quads, s_magic), fd_s(nseg, s_magic);
+            for (int i = tid; i < K * nseg * quads; i += kFlexThreads) {
+                const int rest = fd_q.div(i), q = i - rest * quads;
+                const int kk = fd_s.div(rest), y0 = (rest - kk * nseg) * rows;
+                int slot = s_ehd[e] + 1 + kk;
+                slot -= slot >= K ? K : 0;
+                periph_expand(p, s_sq + slot * pp, q, y0, min(p.S_h, y0 + rows), s_tile + (kk * p.S_h + y0) * quads + q, quads);
+            }
+        } else if (worker && VARIANT != AGYM_OUT_RESIZE_FOV) {   // zero frame (everything outside the window stays zero)
             const uint4 z4 = make_uint4(0u, 0u, 0u, 0u);
             for (int i = tid; i < (tile_bytes >> 4); i += kFlexThreads) reinterpret_cast<uint4 *>(s_tile)[i] = z4;
         }
@@ -651,11 +791,11 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
                               oh, ow, kc, tid, s_magic);
             } else if (blur) {
                 switch (th) {
-                    case 3: flex_hpass<3>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
-                    case 4: flex_hpass<4>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
-                    case 5: flex_hpass<5>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
-                    case 6: flex_hpass<6>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
-                    default: flex_hpass<0>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
+                    case 3: flex_hpass<3, kPeriph>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
+                    case 4: flex_hpass<4, kPeriph>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
+                    case 5: flex_hpass<5, kPeriph>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
+                    case 6: flex_hpass<6, kPeriph>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
+                    default: flex_hpass<0, kPeriph>(g, s_t1, s_wh2, s_xh, s_tile, k0, kc, th, tid, s_magic); break;
                 }
             } else {
                 const FastDiv fd_nq(g.nq, s_magic), fd_rh(rh, s_magic);
@@ -663,7 +803,14 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
                 for (int i = tid; i < kc * rh * g.nq; i += kFlexThreads) {
                     const int row = fd_nq.div(i), q = i - row * g.nq;
                     const int kk = fd_rh.div(row), y = row - kk * rh;
-                    if (y < g.vh) s_tile[((k0 + kk) * oh + oy + y) * g.ow4 + g.wlo + q] = t1w[i];
+                    if (y >= g.vh) continue;
+                    uint32_t *d = s_tile + ((k0 + kk) * oh + oy + y) * g.ow4 + g.wlo + q;
+                    if (kPeriph) {   // the edge words keep the background's bytes (t1w is zero outside the window)
+                        const uint32_t m = (q == 0 ? g.m_first : 0xffffffffu) & (q == g.nq - 1 ? g.m_last : 0xffffffffu);
+                        *d = (*d & ~m) | t1w[i];
+                    } else {
+                        *d = t1w[i];
+                    }
                 }
             }
         }
@@ -701,10 +848,10 @@ __global__ void __launch_bounds__(kFlexThreads + 32, 2) k_observe_flexible_v3(co
 }  // namespace
 
 // --------------------------------------------------------------------------- launchers
-cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const int32_t *head, const double *action,
-                                    const int32_t *atype, const uint8_t *ctrl, int32_t *loc, int32_t *res, int variant,
-                                    int pad_h, int pad_w, uint8_t *out, int32_t *err, void *norm_out, int norm_dt,
-                                    cudaStream_t st) {
+cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const int32_t *head, const float *pcache,
+                                    const double *action, const int32_t *atype, const uint8_t *ctrl, int32_t *loc,
+                                    int32_t *res, int variant, int pad_h, int pad_w, uint8_t *out, int32_t *err,
+                                    void *norm_out, int norm_dt, cudaStream_t st) {
     cudaError_t e;
     DevPlan q = p;
     q.err = err;
@@ -716,19 +863,22 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
         if (out_bytes % 16 != 0) return cudaErrorInvalidValue;
         return launch_normalize(out, out_bytes, norm_dt, norm_out, st);
     };
-    const bool glimpse = variant == AGYM_OUT_RESIZE_FOV;
-    if (variant != AGYM_OUT_RESIZE_FULL && p.flexb && p.flexq && !g_disable_std && !g_flex_old) {
+    const bool glimpse = variant == AGYM_OUT_RESIZE_FOV, periph = variant == kOutPeriph;
+    // the peripheral variant's squeeze arrives by one bulk copy per env and is expanded by the two-tap tables
+    const size_t sq_bytes = periph ? 4 * (size_t)p.K * p.p_h * p.p_w : 0;
+    const bool periph_ok = !periph || (p.fast_expand && sq_bytes % 16 == 0 && (reinterpret_cast<uintptr_t>(pcache) & 15) == 0);
+    if (variant != AGYM_OUT_RESIZE_FULL && p.flexb && p.flexq && periph_ok && !g_disable_std && !g_flex_old) {
         // persistent kernel, 2 CTAs per SM: whatever the fixed buffers leave of ~113 KB goes to t1
         const int oh = variant == AGYM_OUT_CROP ? pad_h : glimpse ? p.f_h : p.S_h;
         const int ow = variant == AGYM_OUT_CROP ? pad_w : glimpse ? p.f_w : p.S_w;
         const size_t tile = (size_t)p.K * oh * ow;
-        const size_t fixed = a16(a16(tile) + 4 * (size_t)p.K * p.S_h * (p.S_w / 4 + 2)) +
+        const size_t fixed = a16(a16(a16(tile) + 4 * (size_t)p.K * p.S_h * (p.S_w / 4 + 2)) + sq_bytes) +
                              4 * ((size_t)p.S_w * 8 + 2 * (size_t)p.S_h * p.blur_tmax + p.S_w + p.S_h) + 16;
         // floats: one / all K frames of the largest window (the glimpse keeps f_w columns of each window row)
         const size_t one = (size_t)p.S_h * (glimpse ? p.f_w : p.S_w + 4), all = (size_t)p.K * one;
         // + static shared memory + 1 KB reserved per CTA: two CTAs per SM (233,472 B).  RGB plans whose fixed buffers do
-        // not leave one window's t1 in that budget (mask_out at 3 frames x 3 planes: 133 KB of tile and strips) run
-        // one CTA per SM with the whole SM's shared memory instead
+        // not leave one window's t1 in that budget (mask_out at 3 frames x 3 planes: 133 KB of tile and strips; the
+        // peripheral variant adds 14,400 B of squeeze) run one CTA per SM with the whole SM's shared memory instead
         const int ctas_per_sm = (p.C == 3 && fixed + 4 * one > 114000) ? 1 : 2;
         const size_t budget = ctas_per_sm == 2 ? 114000 : 225000;
         const size_t room = budget > fixed ? ((budget - fixed) / 4) & ~size_t(3) : 0;
@@ -751,13 +901,16 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
             if ((e = cudaMemsetAsync(p.flex_counters, 0, 16, st)) != cudaSuccess) return e;
             if (variant == AGYM_OUT_CROP) {
                 if ((e = set_smem(k_observe_flexible_v3<AGYM_OUT_CROP>, fs)) != cudaSuccess) return e;
-                k_observe_flexible_v3<AGYM_OUT_CROP><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, 0);
+                k_observe_flexible_v3<AGYM_OUT_CROP><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, 0, nullptr);
+            } else if (periph) {
+                if ((e = set_smem(k_observe_flexible_v3<kOutPeriph>, fs)) != cudaSuccess) return e;
+                k_observe_flexible_v3<kOutPeriph><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, 0, pcache);
             } else if (glimpse) {
                 if ((e = set_smem(k_observe_flexible_v3<AGYM_OUT_RESIZE_FOV>, fs)) != cudaSuccess) return e;
-                k_observe_flexible_v3<AGYM_OUT_RESIZE_FOV><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, bulk_out ? 0 : 1);
+                k_observe_flexible_v3<AGYM_OUT_RESIZE_FOV><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, bulk_out ? 0 : 1, nullptr);
             } else {
                 if ((e = set_smem(k_observe_flexible_v3<AGYM_OUT_MASK>, fs)) != cudaSuccess) return e;
-                k_observe_flexible_v3<AGYM_OUT_MASK><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, 0);
+                k_observe_flexible_v3<AGYM_OUT_MASK><<<grid, kFlexThreads + 32, fs, st>>>(q, ring, head, action, atype, ctrl, loc, res, oh, ow, (int)t1_cap, out, p.flex_counters, 0, nullptr);
             }
             return cudaGetLastError();
         }
@@ -780,11 +933,14 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
             return finish(cudaGetLastError());
         }
     }
-    const size_t smem = sizeof(float) * 2 * (size_t)p.plane;
+    // window buffers; the peripheral variant adds the background plane and, for generic expand tables, squeeze + W pass
+    const size_t smem = sizeof(float) * 2 * (size_t)p.plane +
+                        (periph ? p.plane + sizeof(float) * ((size_t)p.p_h * p.p_w + (size_t)p.p_h * p.S_w) : 0);
 #define AGYM_LAUNCH_FLEX(V)                                                                              \
     if ((e = set_smem(k_observe_flexible<V>, smem)) != cudaSuccess) return e;                            \
-    k_observe_flexible<V><<<p.N, kThreads, smem, st>>>(q, ring, head, action, atype, ctrl, loc, res, pad_h, pad_w, out);
-    if (variant == AGYM_OUT_CROP) { AGYM_LAUNCH_FLEX(AGYM_OUT_CROP) }
+    k_observe_flexible<V><<<p.N, kThreads, smem, st>>>(q, ring, head, action, atype, ctrl, loc, res, pad_h, pad_w, out, pcache);
+    if (periph) { AGYM_LAUNCH_FLEX(kOutPeriph) }
+    else if (variant == AGYM_OUT_CROP) { AGYM_LAUNCH_FLEX(AGYM_OUT_CROP) }
     else if (variant == AGYM_OUT_MASK) { AGYM_LAUNCH_FLEX(AGYM_OUT_MASK) }
     else if (glimpse) { AGYM_LAUNCH_FLEX(AGYM_OUT_RESIZE_FOV) }
     else { AGYM_LAUNCH_FLEX(AGYM_OUT_RESIZE_FULL) }

@@ -101,10 +101,12 @@ cudaError_t launch_observe_fixed(const DevPlan &p, const uint8_t *ring, const in
 cudaError_t launch_observe_peripheral(const DevPlan &p, const ExpandStd *ew, const uint8_t *ring, const int32_t *head,
                                       const float *pcache, const double *action, const uint8_t *ctrl, int32_t *loc,
                                       uint8_t *out, void *norm_out, int norm_dt, cudaStream_t st);
-cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const int32_t *head, const double *action,
-                                    const int32_t *atype, const uint8_t *ctrl, int32_t *loc, int32_t *res, int variant,
-                                    int pad_h, int pad_w, uint8_t *out, int32_t *err, void *norm_out, int norm_dt,
-                                    cudaStream_t st);
+// variant: AGYM_OUT_* or kOutPeriph; pcache: the squeeze cache kOutPeriph expands (null otherwise)
+constexpr int kOutPeriph = 4;   // flexible fovea over the peripheral background (agym_observe_flexible_peripheral)
+cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const int32_t *head, const float *pcache,
+                                    const double *action, const int32_t *atype, const uint8_t *ctrl, int32_t *loc,
+                                    int32_t *res, int variant, int pad_h, int pad_w, uint8_t *out, int32_t *err,
+                                    void *norm_out, int norm_dt, cudaStream_t st);
 cudaError_t launch_normalize(const uint8_t *src, size_t n, int dtype, void *dst, cudaStream_t st);
 cudaError_t launch_synth(uint8_t *dst, size_t n, uint64_t seed, cudaStream_t st);
 cudaError_t launch_record_step(int n, int is_reset, const double *raw_reward, const uint8_t *done, const uint8_t *reset_mask,

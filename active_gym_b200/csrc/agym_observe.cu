@@ -432,11 +432,7 @@ __global__ void __launch_bounds__(kThreads) k_observe_peripheral(const __grid_co
 }
 
 // Fast peripheral observe (cached squeeze, bilinear-upsample expand): both expand passes are
-// two-tap lerps r = b + w0 * (a - b).  The cached squeeze is biased by 49152.5 on load; lerp
-// weights sum to one, so the bias rides through both passes and the rounded pixel
-// floor(v + 0.5) ends up in byte 1 of the float's bit pattern (ulp there is 2^-8, so the total
-// evaluation error is < 0.01 u8 LSB) — no float->int conversion, one PRMT tree per 4 pixels.
-constexpr float kBias = 49152.5f;
+// two-tap lerps r = b + w0 * (a - b).  The cached squeeze is biased by kBias on load (see agym_device.cuh).
 
 
 // Persistent CTAs (a few per SM) walk the env batch.  Per env:

@@ -133,3 +133,10 @@ def DMCFixedFovealPeripheralEnv(args, num_envs: Optional[int] = None, source=Non
     from .fov_env import FixedFovealPeripheralEnv, SingleEnvAdapter
     env = FixedFovealPeripheralEnv(DMCBaseEnv(args, num_envs or 1, source, device), args)
     return SingleEnvAdapter(env) if num_envs is None else env
+
+
+def DMCFlexibleFovealPeripheralEnv(args, num_envs: Optional[int] = None, source=None, device=None):
+    """Superset: the flexible fovea over the peripheral background (fov_env.FlexibleFovealPeripheralEnv)."""
+    from .fov_env import FlexibleFovealPeripheralEnv, SingleEnvAdapter
+    env = FlexibleFovealPeripheralEnv(DMCBaseEnv(args, num_envs or 1, source, device), args)
+    return SingleEnvAdapter(env) if num_envs is None else env

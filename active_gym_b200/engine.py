@@ -140,6 +140,13 @@ class ObservationPath:
         t = t.reshape(self.n_envs, 2)
         return t.to(device=self.device, dtype=torch.float64, non_blocking=True).contiguous()
 
+    def _dev_atype(self, action_type) -> Optional[torch.Tensor]:
+        """(N,) FOV_LOC / FOV_RES action types -> int32 device tensor (None: every env FOV_LOC)."""
+        if action_type is None:
+            return None
+        at = torch.as_tensor(np.asarray(action_type) if not isinstance(action_type, torch.Tensor) else action_type)
+        return at.reshape(self.n_envs).to(device=self.device, dtype=torch.int32, non_blocking=True).contiguous()
+
     def raw_frame_shape(self) -> Tuple[int, ...]:
         h, w, c = self.raw_shape
         return (self.n_envs, h, w) if c == 1 else (self.n_envs, h, w, 3)
@@ -214,7 +221,7 @@ class ObservationPath:
 
     def out_shape(self, kind: str, variant: str, pad: Optional[Tuple[int, int]] = None) -> Tuple[int, ...]:
         NK, S = (self.n_envs,) + self._frame_axes(), self.obs_size
-        if kind == "peripheral" or variant in ("mask", "resize_full"):
+        if kind in ("peripheral", "flexible_peripheral") or variant in ("mask", "resize_full"):
             return NK + S
         if kind == "flexible" and variant == "resize_fov":   # the glimpse: every window resampled to fov_size
             return NK + self.fov_size
@@ -275,10 +282,7 @@ class ObservationPath:
         """FlexibleFovealEnv._fov_step + _get_fov_state (fov_env.py:270-330)."""
         ctrl_t = self._ctrl(ctrl)
         act = None if action is None else self._dev_action(action)
-        at = None
-        if action_type is not None:
-            at = torch.as_tensor(np.asarray(action_type) if not isinstance(action_type, torch.Tensor) else action_type)
-            at = at.reshape(self.n_envs).to(device=self.device, dtype=torch.int32, non_blocking=True).contiguous()
+        at = self._dev_atype(action_type)
         pad = tuple(pad) if pad is not None else self.obs_size
         if out is None:
             out = torch.empty(self.out_shape("flexible", variant, pad), dtype=torch.uint8, device=self.device)
@@ -288,6 +292,26 @@ class ObservationPath:
                                                      _ptr(ctrl_t), _ptr(self.loc), _ptr(self.res), VARIANTS[variant],
                                                      int(pad[0]), int(pad[1]), _ptr(out), _ptr(self.err), np_, nd, self._stream()),
                        "agym_observe_flexible")
+        return out
+
+    def observe_flexible_peripheral(self, action, action_type=None, ctrl=None, out: Optional[torch.Tensor] = None,
+                                    norm_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The flexible fovea over the peripheral background: FlexibleFovealEnv._fov_step (fov_env.py:300-330), then
+        FixedFovealPeripheralEnv's observation (fov_env.py:366-368, 376, 385-386) with the window, blurred iff
+        rh > f_h, pasted at its flexible place.  Needs the squeeze cache (``cache_peripheral=True``)."""
+        if self.pcache is None:
+            raise ValueError("observe_flexible_peripheral needs the squeeze cache: build the path with cache_peripheral=True")
+        ctrl_t = self._ctrl(ctrl)
+        act = None if action is None else self._dev_action(action)
+        at = self._dev_atype(action_type)
+        if out is None:
+            out = torch.empty(self.out_shape("flexible_peripheral", "mask"), dtype=torch.uint8, device=self.device)
+        np_, nd = self._norm(out, norm_out)
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.agym_observe_flexible_peripheral(
+                self._plan, _ptr(self.ring), _ptr(self.head), _ptr(self.pcache), _ptr(act), _ptr(at), _ptr(ctrl_t),
+                _ptr(self.loc), _ptr(self.res), _ptr(out), _ptr(self.err), np_, nd, self._stream()),
+                "agym_observe_flexible_peripheral")
         return out
 
     def read_errors(self) -> int:

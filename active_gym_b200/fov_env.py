@@ -422,6 +422,44 @@ class FixedFovealPeripheralEnv(FixedFovealEnv):
         return self.path.observe_peripheral(action, ctrl=ctrl, out=self._out, host_out=self.host_obs, norm_out=norm_out)
 
 
+class FlexibleFovealPeripheralEnv(FlexibleFovealEnv):
+    """Superset (the reference has no such wrapper): ``FlexibleFovealEnv`` whose background is
+    ``FixedFovealPeripheralEnv``'s periphery instead of ``mask_out``'s zeros.  Per env, after this step's fovea update
+    (fov_env.py:300-330, unchanged, FOV_RES checks included), each plane of the stack is
+    ``Resize(obs_size)(Resize(peripheral_res)(full))`` (fov_env.py:366-368, 376) with the window
+    ``full[r:r+rh, c:c+rw]`` pasted at its place (fov_env.py:385-386), blurred by ``Resize(fov_res)(Resize(fov_size)(.))``
+    iff ``rh > f_h`` (fov_env.py:276-280, 286-287).  Observation: uint8 (N, K, S_h, S_w), or (N, K, 3, S_h, S_w) for RGB;
+    ``info`` carries ``fov_loc`` and ``fov_res``; the action space is the flexible one.
+
+    Like the reference's peripheral constructor (fov_env.py:361) it forces ``mask_out = False``.  ``resize_to_fov``
+    selects a different observation and raises ``ValueError``, as do a ``peripheral_res`` other than the base env's and
+    a base env built with ``cache_peripheral=False`` (the kernels expand the squeeze cache the ingest keeps)."""
+
+    _kind = "flexible_peripheral"
+
+    def __init__(self, env, args):
+        if bool(getattr(args, "resize_to_fov", False)):
+            raise ValueError("resize_to_fov selects the glimpse; FlexibleFovealPeripheralEnv returns full frames")
+        super().__init__(env, args)
+        self.mask_out = False
+        self.peripheral_res = tuple(args.peripheral_res)
+        self.observation_space = Box(low=-1., high=1., shape=self._frame_axes() + tuple(self.obs_size), dtype=np.float32)
+        if self.path.peripheral_res != self.peripheral_res:
+            raise ValueError("the base env was built from different args (peripheral_res mismatch)")
+        if self.path.pcache is None:
+            raise ValueError("FlexibleFovealPeripheralEnv needs the squeeze cache: build the base env with cache_peripheral=True")
+
+    @property
+    def variant(self) -> str:
+        return "mask"   # full frames: the output shape of mask_out
+
+    def _observe(self, action, ctrl, action_type=None, norm_out=None):
+        self._check_res(action, action_type)
+        self._device_actions = isinstance(action, torch.Tensor) and action.device.type == "cuda"
+        return self.path.observe_flexible_peripheral(action, action_type, ctrl=ctrl, out=self._out, host_out=self.host_obs,
+                                                     norm_out=norm_out)
+
+
 class SingleEnvAdapter:
     """The N=1 drop-in: presents a batched env with the reference's single-env types — float64
     NumPy observations normalised to [0,1] (= float32(u8)/255), scalar reward / done, NumPy

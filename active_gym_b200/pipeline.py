@@ -385,6 +385,7 @@ class PipelinedPath:
         else:
             ct = self._small_to_device("ctrl", ctrl, torch.uint8, None)
         h_obs = h_loc = None
+        flex = kind in ("flexible", "flexible_peripheral")   # fov_res travels with the observation
         if host_out:
             hk = (kind, variant, tuple(shape))
             if hk not in self._h_out:
@@ -398,16 +399,18 @@ class PipelinedPath:
                 p.observe_peripheral(a, ctrl=c, out=out[lo:hi], norm_out=nrm)
             elif kind == "flexible":
                 p.observe_flexible(a, None if at is None else at[i], variant=variant, ctrl=c, pad=pad, out=out[lo:hi], norm_out=nrm)
+            elif kind == "flexible_peripheral":
+                p.observe_flexible_peripheral(a, None if at is None else at[i], ctrl=c, out=out[lo:hi], norm_out=nrm)
             else:
                 p.observe_fixed(a, variant=variant, ctrl=c, out=out[lo:hi], norm_out=nrm)
             if host_out:
                 h_obs[lo:hi].copy_(out[lo:hi], non_blocking=True)
                 h_loc[lo:hi].copy_(self.loc[lo:hi], non_blocking=True)
-                if kind == "flexible":
+                if flex:
                     h_res[lo:hi].copy_(self.res[lo:hi], non_blocking=True)
         if host_out:
-            self.d2h_bytes += h_obs.numel() + h_loc.numel() * 4 * (2 if kind == "flexible" else 1)
-            return out, (h_obs, h_loc, h_res if kind == "flexible" else None)
+            self.d2h_bytes += h_obs.numel() + h_loc.numel() * 4 * (2 if flex else 1)
+            return out, (h_obs, h_loc, h_res if flex else None)
         self.join()
         return out
 
@@ -428,6 +431,13 @@ class PipelinedPath:
         """FlexibleFovealEnv._fov_step + _get_fov_state (fov_env.py:270-330)."""
         pad = tuple(pad) if pad is not None else self.obs_size
         return self._observe("flexible", action, action_type, variant, ctrl, pad, out, host_out, norm_out)
+
+    def observe_flexible_peripheral(self, action, action_type=None, ctrl=None, out=None, host_out: bool = False,
+                                    norm_out=None):
+        """The flexible fovea over the peripheral background (ObservationPath.observe_flexible_peripheral)."""
+        if self.pcache is None:
+            raise ValueError("observe_flexible_peripheral needs the squeeze cache: build with cache_peripheral=True")
+        return self._observe("flexible_peripheral", action, action_type, "mask", ctrl, None, out, host_out, norm_out)
 
     def record_step(self, raw_reward=None, done=None, reset_mask=None, is_reset: bool = False,
                     trace_row: Optional[torch.Tensor] = None, with_res: bool = False, host_out: bool = False):

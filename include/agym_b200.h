@@ -200,6 +200,24 @@ AGYM_API int agym_observe_flexible(const agym_plan *plan, const uint8_t *d_ring,
                           int32_t *d_loc, int32_t *d_res, int variant, int pad_h, int pad_w,
                           uint8_t *d_out, int32_t *d_err, void *d_out_norm, int norm_dtype, void *stream);
 
+/* The flexible fovea over a peripheral background (a superset of the reference, which has no such wrapper):
+ * FlexibleFovealEnv._fov_step (fov_env.py:300-330, with the same d_atype, d_fov_ctrl, d_res and d_err semantics as
+ * agym_observe_flexible) followed by FixedFovealPeripheralEnv's observation (fov_env.py:366-368, 376, 385-386) with the
+ * window pasted at its flexible size and place.  Per plane: bg = Resize(obs_size)(Resize(peripheral_res)(full)) from
+ * the squeeze cache d_pcache (f32 [N][P][p_h][p_w], kept by the ingest calls; required); the window
+ * full[r:r+rh, c:c+rw] is blurred by Resize(fov_res)(Resize(fov_size)(win)) iff rh > f_h (fov_env.py:276-280, 286-287)
+ * and written over bg.  d_out: u8 [N][P][S_h][S_w], P = frame_stack * C.
+ * Window pixels are bit for bit those of agym_observe_flexible(AGYM_OUT_MASK) on the same state (so bit exact when not
+ * blurred, within 0.5 LSB + 0.02 of the reference's float value when blurred); background pixels are within 0.5 LSB +
+ * 0.01 of it, and bit for bit agym_observe_peripheral's where that call runs its standard-geometry kernel (grey, 84x84
+ * observations, 20x20 periphery).  Any d_out alignment is served (the fast kernel needs 16 bytes).
+ * AGYM_ERR_INVALID_ARG for a plan without a fovea or a periphery and for NULL d_pcache or d_res.  Added without an ABI
+ * version bump: the struct and every other signature are unchanged. */
+AGYM_API int agym_observe_flexible_peripheral(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head,
+                          const float *d_pcache, const double *d_action, const int32_t *d_atype,
+                          const uint8_t *d_fov_ctrl, int32_t *d_loc, int32_t *d_res, uint8_t *d_out,
+                          int32_t *d_err, void *d_out_norm, int norm_dtype, void *stream);
+
 /* Replaces RecordWrapper's episode counters (fov_env.py:15-67) and the fov_loc / fov_res trace that
  * save_transition keeps when record=True (fov_env.py:152-154, 205-207, 253-256, 332-335), for N envs on the device.
  *   step  (is_reset = 0): ep_len += 1; cum_reward += d_raw_reward (f64 [N], info["raw_reward"]; NULL = 0)

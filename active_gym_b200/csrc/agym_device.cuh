@@ -285,6 +285,9 @@ __device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
 }
 // barrier among the consumer warps only (the producer warp never joins it)
 __device__ __forceinline__ void consumer_sync() { asm volatile("bar.sync 1, %0;" ::"n"(kThreads) : "memory"); }
+// barrier among the THREADS threads (whole warps) that share named barrier `id` (1..15; 0 is __syncthreads)
+template <int THREADS>
+__device__ __forceinline__ void named_sync(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(THREADS) : "memory"); }
 
 // ---- programmatic dependent launch (PDL).  A kernel launched through launch_pdl() may start while the kernel before
 // it in the stream is still draining: pdl_launch_dependents() (first statement of every such kernel) lets the NEXT

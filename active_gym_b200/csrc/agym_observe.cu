@@ -624,23 +624,32 @@ __global__ void __launch_bounds__(128) k_observe_peripheral_v2(const __grid_cons
 // immediate offsets, no index arithmetic.  The plan checks the host tables against this pattern
 // before the kernel is used; the WEIGHTS always come from the host tables (ATen's values).
 //
-// One thread = one 4-pixel column quad q of one frame k over one 21-row segment g (21 x K x 4
-// threads per env).  It W-expands the 7 squeezed rows it needs straight from the cached squeeze
+// One thread = one 4-pixel column quad q of one frame k over one 21-row segment g (21 x 4 threads
+// per plane).  It W-expands the 7 squeezed rows it needs straight from the cached squeeze
 // in shared memory — three adjacent samples s0..s2 cover its four columns, so
 //   T[c] = a[c] * s0 + b[c] * s1 + g[c] * s2 + bias      (one of a[c], g[c] is zero)
 // is 6 FFMA2 per row with per-thread constant weights — then H-expands, quantises, pastes the
-// fovea and stores one word per row: 2 FFMA2 + 3 PRMT + (LDS + LOP3 on fovea rows) + 1 STG.
+// fovea and stores one word per row: 2 FFMA2 + 3 PRMT + (LDS + LOP3 on fovea rows) + 1 STS.
 // The bias 49152.5 puts the rounded pixel floor(v + 0.5) into byte 1 of the float (ulp 2^-8,
 // total evaluation error < 0.01 u8 LSB), so there is no float->int conversion.
-// Persistent CTAs, one block-wide barrier per env.  Inputs run two envs ahead through three
-// shared-memory buffers: for env e+2 one elected thread issues a single TMA bulk copy
-// (cp.async.bulk, completion on an mbarrier) of the env's cached squeeze (K x 400 f32, contiguous),
-// and every thread cp.asyncs exactly the ring words it will itself paste (same (row, quad) as its
-// output words: immediate offsets, no index arithmetic).  Outputs are assembled in a
-// double-buffered shared-memory tile and leave as ONE TMA bulk store per env (28,224 contiguous
-// bytes) — 4-byte stores straight to global ran the write path at 40 % of HBM bandwidth.
-// Every 32 iterations warp 0 applies the sensory actions of the CTA's next 32 envs to fov_loc,
-// one env per lane (fov_env.py:187-199).
+//
+// Persistent CTAs of K plane groups: group k (3 warps, 96 threads, 84 of them computing) produces
+// frame k of every env of the CTA and runs its own pipeline, synchronised by its own named barrier —
+// there is no CTA-wide barrier in the env loop, so a thread waits only for the 95 others that share
+// its plane and a group may run ahead of the others by the depth of its own buffers.  Per group:
+//   - inputs run two envs ahead through three shared-memory buffers: for env e+2 the group's
+//     leader issues one TMA bulk copy (cp.async.bulk, completion on the group's own mbarrier) of the
+//     plane's cached squeeze (400 f32), and the group stages its plane's fovea bytes itself (below),
+//     so the copies it waits for are its own;
+//   - the plane is assembled in a double-buffered 7,056-byte tile and leaves as ONE TMA bulk store
+//     to out + e * 28,224 + k * 7,056 (4-byte stores straight to global ran the write path at 40 %
+//     of HBM bandwidth); the leader issues, commits and waits its group's bulk groups, which are
+//     per thread, so the groups do not interfere.
+// The sensory actions: every 32 iterations warp 0 applies those of the CTA's next 32 envs to fov_loc,
+// one env per lane (fov_env.py:187-199), into a ring of four 32-entry batches.  A batch is published
+// on its `loc_full` mbarrier (the groups wait for it before they prefetch its first env) and handed
+// back on its `loc_free` mbarrier (each group's leader arrives once the group has left the batch), so
+// warp 0 rewrites a slot only after every group has passed it, however far apart the groups run.
 struct StdGeom {
     static constexpr int S = 84, P = 20, Q = 21, SEG = 4, R = 21, SPAN = 7;
     // floor((40 i - 64) / 168): source index of output i relative to the 20-sample axis
@@ -659,34 +668,42 @@ __device__ __forceinline__ void prefetch_rows_imm(uint32_t rows, uint32_t dst, c
 // FS ("full-row staging"): the sharp fovea bytes are staged as 16-byte chunks at the positions they have in the ring
 // (the staging buffer of a frame mirrors the ring words [lr * 21 & ~3, ...) of its slot, so a chunk copy is aligned on
 // both sides and the paste reads word (row r, quad q) at an immediate offset).  Only the chunks that meet the fovea
-// columns are copied: K * f_h * 3 copies of 16 bytes per env, about one per thread and a dozen instructions each,
-// instead of up to 21 predicated 4-byte copies per thread (a quarter of the kernel's instructions).  Costs 2.5 KB of
-// shared memory per frame and buffer; used when two CTAs still fit an SM (the standard 30x30 fovea does).
+// columns are copied: f_h * 3 copies of 16 bytes per plane, about one per thread of the plane's group and a dozen
+// instructions each, instead of up to 21 predicated 4-byte copies per thread (a quarter of the kernel's instructions).
+// A chunk is pasted by other threads than the one that copied it, so each group copies its own plane's chunks and
+// waits for them before its own barrier.  Costs 2.5 KB of shared memory per frame and buffer; used when two CTAs
+// still fit an SM (the standard 30x30 fovea does).
 template <int K, int NW, bool FS>  // NW: words per staged fovea row, (f_w + 3) / 4 + 1, when baked in; 0 = from the plan
-__global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 32, 2)
+__global__ void __launch_bounds__(96 * K, 2)
     k_observe_peripheral_std(const __grid_constant__ DevPlan p, const __grid_constant__ ExpandStd ew,
                              const uint8_t *__restrict__ ring, const int32_t *__restrict__ head,
                              const float *__restrict__ pcache, const double *__restrict__ action,
                              const uint8_t *__restrict__ ctrl, int32_t *__restrict__ loc, uint8_t *__restrict__ out) {
     using Gm = StdGeom;
     constexpr int S = Gm::S, P = Gm::P, Q = Gm::Q, R = Gm::R;
-    constexpr int NB = Q * Gm::SEG * K;
+    constexpr int GT = 96;  // threads of one plane group
     constexpr int PP = P * P, PLANE_W = S * S / 4;
-    constexpr int NBUF = 3, DIST = 2, LOC_RING = 128;
+    constexpr int NBUF = 3, DIST = 2, LOC_RING = 128, LOC_BATCHES = LOC_RING / 32;
     extern __shared__ __align__(16) uint8_t smem[];
     __shared__ int4 s_loc[LOC_RING];  // {fov row, fov col, head, -} of the CTA's iteration j at [j % LOC_RING]
-    __shared__ __align__(8) uint64_t full[NBUF];
+    __shared__ __align__(8) uint64_t full[K][NBUF];
+    __shared__ __align__(8) uint64_t loc_full[LOC_BATCHES], loc_free[LOC_BATCHES];
     const int tid = threadIdx.x;
+    const int k = tid / GT, lt = tid - k * GT;  // plane group = frame k of the stack; thread lt of the group
+    const bool lead = lt == 0;
     const int N = p.N, f_h = p.f_h, f_w = p.f_w, G = gridDim.x;
     const int nw_max = NW ? NW : (f_w + 3) / 4 + 1;
-    const int rowbuf = (f_h * Q + 9) & ~3;          // FS: staged words of one frame (alignment slack on both sides)
-    const int buf_words = K * PP + (FS ? K * rowbuf : ((K * f_h * nw_max + 3) & ~3));
-    float *bufs = reinterpret_cast<float *>(smem);  // [NBUF]{ sq [K slots][P][P] | fov [K][f_h][nw_max] or [K][rowbuf] }
-    uint32_t *tiles = reinterpret_cast<uint32_t *>(bufs + NBUF * buf_words);  // [2][K][S][S / 4] output words
+    const int rowbuf = (f_h * Q + 9) & ~3;  // FS: staged words of one frame (alignment slack on both sides)
+    const int buf_words = PP + (FS ? rowbuf : ((f_h * nw_max + 3) & ~3));
+    // the group's shared memory: [NBUF]{ sq [P][P] | fov [f_h][nw_max] or [rowbuf] }, then [2][S][S / 4] output words
+    float *bufs = reinterpret_cast<float *>(smem) + k * (NBUF * buf_words + 2 * PLANE_W);
+    uint32_t *tiles = reinterpret_cast<uint32_t *>(bufs + NBUF * buf_words);
     const uint32_t *ring_w = reinterpret_cast<const uint32_t *>(ring);
 
     // fov_loc (after this step's action) and head of iterations [it0, it0 + 32), one per lane (warp 0)
     auto loc_batch = [&](int it0) {
+        const int bt = it0 / 32;
+        if (bt >= LOC_BATCHES) mbar_wait(&loc_free[bt % LOC_BATCHES], (bt / LOC_BATCHES - 1) & 1);  // every group left bt - 4
         const int j = it0 + (tid & 31);
         // j * G cannot overflow: a CTA runs at most N / G + 1 iterations and batches reach 64 past that
         const int env = j <= N / G + 1 ? (int)blockIdx.x + j * G : N;
@@ -696,22 +713,22 @@ __global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 
             hh = head[env];
         }
         s_loc[j & (LOC_RING - 1)] = make_int4(r, c, hh, 0);
+        mbar_arrive(&loc_full[bt % LOC_BATCHES]);
     };
     pdl_launch_dependents();
     if (tid == 0) {
-        for (int i = 0; i < NBUF; ++i) mbar_init(&full[i], 1);
+        for (int i = 0; i < K * NBUF; ++i) mbar_init(&full[i / NBUF][i % NBUF], 1);
+        for (int i = 0; i < LOC_BATCHES; ++i) {
+            mbar_init(&loc_full[i], 32);
+            mbar_init(&loc_free[i], K);
+        }
         mbar_fence_init();
     }
 
-    const bool active = tid < NB;
-    const int q = tid % Q, t2 = tid / Q;
-    // which (frame, segment) group the t2-th run of 21 threads works on: an order found by search that keeps
-    // the two or three groups sharing a warp on different shared-memory banks when they store their tile words
-    // (word offset 1764 k + 441 g + 21 r + q); in k-major order every warp's stores were 2-way conflicts
-    constexpr int kOrd4[16] = {7, 4, 13, 3, 0, 1, 9, 6, 10, 14, 11, 12, 8, 5, 15, 2};
-    constexpr int kOrd3[12] = {11, 8, 5, 2, 9, 6, 3, 0, 10, 4, 1, 7};
-    const int grp = !active ? 0 : (K == 4 ? kOrd4[t2 & 15] : (K == 3 ? kOrd3[t2 % 12] : t2));
-    const int g = grp % Gm::SEG, k = grp / Gm::SEG;
+    const bool active = lt < Q * Gm::SEG;
+    // segment order 3, 0, 1, 2 over the group's runs of 21 threads: of the tile stores (word 441 g + 21 r + q), only
+    // the middle warp's are 2-way bank conflicts; in order 0..3 two of the three warps had them
+    const int q = lt % Q, g = (lt / Q + 3) & 3;
     // W pass: samples base .. base + 2 of a squeezed row cover this quad's columns
     int base;
     uint64_t wa01, wa23, wb01, wb23, wc01, wc23;  // weights of s0 / s1 / s2 for columns (0,1) and (2,3)
@@ -732,24 +749,23 @@ __global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 
         wc01 = pack2(wc[0], wc[1]); wc23 = pack2(wc[2], wc[3]);
     }
     const uint64_t bias2 = pack2(kBias, kBias);
-    // squeezed rows 5g-1 .. 5g+5, clamped to the frame: float offsets inside one staged slot
+    // squeezed rows 5g-1 .. 5g+5, clamped to the frame: float offsets inside one staged squeeze
     const int row_first = 5 * g - 1;
     const int so_t0 = (row_first < 0 ? 0 : row_first) * P + base;                 // t = 0
     const int so_mid = row_first * P + base;                                      // t = 1..5 at + t * P
     const int so_t6 = (row_first + 6 > P - 1 ? P - 1 : row_first + 6) * P + base;  // t = 6
     const uint32_t bufs_s = smem_u32(bufs);
     const uint32_t word0 = (uint32_t)(g * R) * Q + q;  // this thread's first output word inside a plane
-    // FS: the (at most two) 16-byte chunks this thread stages for every env: chunk c of fovea row y of frame k
+    // FS: the (at most two) 16-byte chunks this thread stages of its plane for every env: chunk c of fovea row y
+    // (the launcher's bound on K * f_h * chunks per row keeps a plane within 2 * 96 chunks)
     constexpr int NJ = 2;
-    int ck_row[NJ], ck_k[NJ], ck_c4[NJ];
+    int ck_row[NJ], ck_c4[NJ];
     if constexpr (FS) {
-        const int cpr = (f_w + 14) / 16 + 1, total = K * f_h * cpr;
+        const int cpr = (f_w + 14) / 16 + 1, total = f_h * cpr;
 #pragma unroll
         for (int a = 0; a < NJ; ++a) {
-            const int i = tid + a * (int)blockDim.x;
-            const int row = i / cpr, kk = row / f_h;
-            ck_k[a] = i < total ? kk : -1;
-            ck_row[a] = (row - kk * f_h) * Q;
+            const int i = lt + a * GT, row = i / cpr;
+            ck_row[a] = i < total ? row * Q : -1;
             ck_c4[a] = (i - row * cpr) * 4;
         }
     }
@@ -762,40 +778,39 @@ __global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 
         return (mask && m_hi > m_lo) ? (((1u << m_hi) - 1u) & ~((1u << m_lo) - 1u)) : 0u;
     };
     // staged position (word index inside a buffer's fovea tile) of this thread's row r = 0
-    auto fovea_pos = [&](int lr, int lc) { return (k * f_h + g * R - lr) * nw_max + (q - (lc >> 2)); };
-    // prefetch for iteration j (env) into buffer j % NBUF
+    auto fovea_pos = [&](int lr, int lc) { return (g * R - lr) * nw_max + (q - (lc >> 2)); };
+    // prefetch of this group's plane for iteration j (env) into buffer j % NBUF
     auto prefetch = [&](int env, int j) {
-        // buffer j % NBUF: its last tenant (iteration j - NBUF) was consumed before the barrier that
-        // ended iteration j - DIST - 1, which every thread has passed
+        // buffer j % NBUF: its last tenant (iteration j - NBUF) was consumed before the group barrier that
+        // ended iteration j - DIST - 1, which every thread of the group has passed
         const int b = j % NBUF;
-        if (tid == 0) {
-            mbar_expect_tx(&full[b], K * PP * 4);
-            bulk_g2s(bufs + b * buf_words, pcache + (size_t)env * (K * PP), K * PP * 4, &full[b]);
+        // s_loc entry j: its batch is published when the group first needs it, at the batch's first entry
+        if ((j & 31) == 0) mbar_wait(&loc_full[(j / 32) % LOC_BATCHES], (j / 32 / LOC_BATCHES) & 1);
+        const int4 lh = s_loc[j & (LOC_RING - 1)];
+        int slot = lh.z + 1 + k;
+        slot -= slot >= K ? K : 0;
+        if (lead) {
+            mbar_expect_tx(&full[k][b], PP * 4);
+            bulk_g2s(bufs + b * buf_words, pcache + ((size_t)env * K + slot) * PP, PP * 4, &full[k][b]);
         }
+        const uint32_t *plane = ring_w + ((size_t)env * K + slot) * PLANE_W;
         if constexpr (FS) {
-            const int4 lh = s_loc[j & (LOC_RING - 1)];
-            const int top = lh.x * Q, wb = top & ~3;           // ring word (inside a plane) the staging buffers start at
+            const int top = lh.x * Q, wb = top & ~3;  // ring word (inside a plane) the staging buffer starts at
             const int lw = lh.y >> 2, lastw = (lh.y + f_w - 1) >> 2;
 #pragma unroll
             for (int a = 0; a < NJ; ++a) {
-                if (ck_k[a] < 0) continue;
+                if (ck_row[a] < 0) continue;
                 const int rowbase = top + ck_row[a];
                 const int cw = ((rowbase + lw) & ~3) + ck_c4[a];  // an aligned chunk that starts inside the plane ends inside it
                 if (cw > rowbase + lastw) continue;
-                int slot = lh.z + 1 + ck_k[a];
-                slot -= slot >= K ? K : 0;
-                cp_async16_s(bufs_s + (uint32_t)(b * buf_words + K * PP + ck_k[a] * rowbuf + (cw - wb)) * 4u,
-                             ring_w + ((size_t)env * K + slot) * PLANE_W + cw);
+                cp_async16_s(bufs_s + (uint32_t)(b * buf_words + PP + (cw - wb)) * 4u, plane + cw);
             }
         } else if (active) {
-            const int4 lh = s_loc[j & (LOC_RING - 1)];
             uint32_t mask;
             const uint32_t rows = fovea_rows(lh.x, lh.y, mask);
             if (rows) {
-                int slot = lh.z + 1 + k;
-                slot -= slot >= K ? K : 0;
-                const uint32_t *src = ring_w + ((size_t)env * K + slot) * PLANE_W + word0;
-                const uint32_t dst = bufs_s + (uint32_t)(b * buf_words + K * PP + fovea_pos(lh.x, lh.y)) * 4u;
+                const uint32_t *src = plane + word0;
+                const uint32_t dst = bufs_s + (uint32_t)(b * buf_words + PP + fovea_pos(lh.x, lh.y)) * 4u;
                 if (NW) {
                     prefetch_rows_imm<NW, 0>(rows, dst, src);
                 } else {
@@ -815,8 +830,8 @@ __global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 
     };
 
     pdl_wait();       // ring, head, pcache, action, loc, out: not before the previous kernel in the stream has finished
+    __syncthreads();  // mbarriers initialised
     if (tid < 32) loc_batch(0);
-    __syncthreads();  // s_loc of the first 32 iterations, mbarriers initialised
     {
         const int e0 = blockIdx.x;
 #pragma unroll
@@ -824,9 +839,9 @@ __global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 
             if (e0 + j * G < N) prefetch(e0 + j * G, j);
             cp_async_commit();
         }
-        if constexpr (FS) {   // chunks are staged by other threads than the ones that paste them
+        if constexpr (FS) {   // the group's chunks of the first env, visible to the whole group after its barrier
             cp_async_wait<DIST - 1>();
-            __syncthreads();
+            named_sync<GT>(1 + k);
         }
     }
     int it = 0;
@@ -836,19 +851,17 @@ __global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 
         if ((it & 31) == 0 && tid < 32) loc_batch(it + 32);
         const int b = it % NBUF;
         if constexpr (!FS) cp_async_wait<DIST>();    // this thread's own fovea words of env e
-        mbar_wait(&full[b], (it / NBUF) & 1);        // the env's cached squeeze (TMA)
-        uint32_t *tile = tiles + (it & 1) * (K * PLANE_W);
+        mbar_wait(&full[k][b], (it / NBUF) & 1);     // the plane's cached squeeze (TMA)
+        uint32_t *tile = tiles + (it & 1) * PLANE_W;
         if (active) {
             const int4 lh = s_loc[it & (LOC_RING - 1)];
             uint32_t fov_mask;
             const uint32_t rows = fovea_rows(lh.x, lh.y, fov_mask);
-            int slot = lh.z + 1 + k;
-            slot -= slot >= K ? K : 0;
-            const float *sq = bufs + b * buf_words + slot * PP;
-            const uint32_t *sh = reinterpret_cast<const uint32_t *>(bufs + b * buf_words + K * PP) +
-                                 (FS ? k * rowbuf + (int)word0 - ((lh.x * Q) & ~3) : fovea_pos(lh.x, lh.y));
+            const float *sq = bufs + b * buf_words;
+            const uint32_t *sh = reinterpret_cast<const uint32_t *>(bufs + b * buf_words + PP) +
+                                 (FS ? (int)word0 - ((lh.x * Q) & ~3) : fovea_pos(lh.x, lh.y));
             constexpr int SHP = FS ? Q : 0;   // staged words between two rows (FS: the ring's own pitch)
-            uint32_t *o = tile + k * PLANE_W + word0;
+            uint32_t *o = tile + word0;
             uint64_t a0, a1, b0, b1, d0 = 0, d1 = 0;
             t_row(sq, so_t0, a0, a1);
             t_row(sq, so_mid + P, b0, b1);
@@ -874,24 +887,25 @@ __global__ void __launch_bounds__(((StdGeom::Q * StdGeom::SEG * K + 31) / 32) * 
                 o[r * Q] = word;
             }
         }
-        // the tile leaves as one TMA store; the store issued two iterations ago has finished reading
-        // this iteration's tile buffer's twin before anyone writes it again (next iteration)
+        // the plane leaves as one TMA store; the store issued one iteration ago has finished reading this
+        // iteration's tile's twin before anyone in the group writes it again (next iteration)
         fence_async_smem();
-        if (tid == 0) bulk_wait_read<0>();
-        if constexpr (FS) cp_async_wait<DIST - 1>();   // this thread's chunks of the NEXT env, visible to all after the barrier
-        __syncthreads();
-        if (tid == 0) {
-            bulk_s2g(out + (size_t)e * (K * PLANE_W * 4), tile, K * PLANE_W * 4);
+        if (lead) bulk_wait_read<0>();
+        if constexpr (FS) cp_async_wait<DIST - 1>();   // this thread's chunks of the NEXT env, visible to the group after the barrier
+        named_sync<GT>(1 + k);
+        if (lead) {
+            if ((it & 31) == 31) mbar_arrive(&loc_free[(it / 32) % LOC_BATCHES]);  // the group is done with this batch
+            bulk_s2g(out + ((size_t)e * K + k) * (PLANE_W * 4), tile, PLANE_W * 4);
             bulk_commit();
         }
-        if (p.norm_out) {   // uniform: the normalised copy of the same tile, 16 pixels per thread and pass; the tile is not
-                            // written again before the barrier of the NEXT iteration, which follows this loop in program order
+        if (p.norm_out) {   // uniform: the normalised copy of the same plane, 16 pixels per thread and pass; the tile is
+                            // not written again before the group barrier of the NEXT iteration
             const uint4 *t4 = reinterpret_cast<const uint4 *>(tile);
-            for (int i = tid; i < K * PLANE_W / 4; i += (int)blockDim.x)
-                norm_store16(p.norm_dt, t4[i], p.norm_out, (size_t)e * (K * PLANE_W / 4) + i);
+            for (int i = lt; i < PLANE_W / 4; i += GT)
+                norm_store16(p.norm_dt, t4[i], p.norm_out, ((size_t)e * K + k) * (PLANE_W / 4) + i);
         }
     }
-    if (tid == 0) bulk_wait_read<0>();  // shared memory must outlive the last store's reads
+    if (lead) bulk_wait_read<0>();  // shared memory must outlive the group's last store's reads
 }
 
 
@@ -977,10 +991,12 @@ cudaError_t launch_observe_peripheral(const DevPlan &p0, const ExpandStd *ew, co
     if (pcache && ew && ew->ok && (p.K == 4 || p.K == 3) && !g_disable_std && p.N < (1 << 30) &&
         (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (reinterpret_cast<uintptr_t>(pcache) & 15) == 0) {  // TMA bulk copies
         const int nw_max = (p.f_w + 3) / 4 + 1;
-        const size_t fov_words = ((size_t)p.K * p.f_h * nw_max + 3) & ~size_t(3);
-        size_t fs = 4 * (3 * ((size_t)p.K * 400 + fov_words) + 2 * (size_t)p.K * 1764);
-        // full-row staging (FS): 16-byte chunk copies; taken when two CTAs still fit an SM and two chunks per thread suffice
-        const size_t fs_rows = 4 * (3 * ((size_t)p.K * 400 + (size_t)p.K * ((p.f_h * 21 + 9) & ~3)) + 2 * (size_t)p.K * 1764);
+        // per plane group: three input buffers { squeeze 400 f32 | staged fovea words } and two 1,764-word output tiles
+        const size_t fov_words = ((size_t)p.f_h * nw_max + 3) & ~size_t(3);
+        size_t fs = 4 * (size_t)p.K * (3 * (400 + fov_words) + 2 * 1764);
+        // full-row staging (FS): 16-byte chunk copies; taken when two CTAs still fit an SM and two chunks per thread
+        // suffice (21 * 4 * K rounded up to warps: at most 176 chunks per plane, within the 2 * 96 of a plane group)
+        const size_t fs_rows = 4 * (size_t)p.K * (3 * (400 + (size_t)((p.f_h * 21 + 9) & ~3)) + 2 * 1764);
         const int std_threads = ((21 * 4 * p.K + 31) / 32) * 32;
         const bool full_rows = !g_std_nofs && fs_rows <= 112 * 1024 && p.K * p.f_h * ((p.f_w + 14) / 16 + 1) <= 2 * std_threads;
         int dev = 0, sms = 148, occ = 0;
@@ -989,7 +1005,7 @@ cudaError_t launch_observe_peripheral(const DevPlan &p0, const ExpandStd *ew, co
 #define AGYM_LAUNCH_STD(KK, NW, FSV)                                                                               \
     {                                                                                                              \
     if (fs <= 220 * 1024) {                                                                                        \
-        const int threads = ((21 * 4 * KK + 31) / 32) * 32;                                                        \
+        const int threads = 96 * KK;   /* one 3-warp group per plane */                                            \
         if ((e = set_smem(k_observe_peripheral_std<KK, NW, FSV>, fs)) != cudaSuccess) return e;                    \
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_observe_peripheral_std<KK, NW, FSV>, threads, fs);   \
         if (occ >= 1) {                                                                                            \

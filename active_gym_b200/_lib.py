@@ -29,7 +29,7 @@ EXPORTS = (
     "agym_plan_ring_bytes", "agym_plan_pcache_bytes", "agym_ingest_atari", "agym_ingest_dmc",
     "agym_stack", "agym_observe_fixed", "agym_observe_peripheral", "agym_observe_flexible",
     "agym_synth_frames", "agym_table_cv2", "agym_table_aa", "agym_table_blur", "agym_normalize", "agym_plan_used_rows", "agym_ingest_atari_packed", "agym_record_step",
-    "agym_observe_flexible_peripheral",
+    "agym_observe_flexible_peripheral", "agym_plan_memory_bytes", "agym_observe_fixed_memory",
 )
 
 
@@ -75,6 +75,9 @@ def lib() -> C.CDLL:
     L.agym_observe_peripheral.argtypes = [vp] * 9 + [i32, vp]
     L.agym_observe_flexible.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, i32, vp]
     L.agym_observe_flexible_peripheral.argtypes = [vp] * 12 + [i32, vp]
+    L.agym_plan_memory_bytes.restype = sz
+    L.agym_plan_memory_bytes.argtypes = [vp, i32]
+    L.agym_observe_fixed_memory.argtypes = [vp] * 6 + [i32] + [vp] * 5 + [i32, vp]
     L.agym_record_step.argtypes = [i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.agym_synth_frames.argtypes = [vp, sz, u64, vp]
     L.agym_normalize.argtypes = [vp, sz, i32, vp, vp]

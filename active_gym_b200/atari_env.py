@@ -37,6 +37,8 @@ class AtariEnvArgs:
         self.resize_to_full = False  # superset: no default in the reference (fov_env.py:120)
         # superset: FlexibleFovealEnv returns the glimpse, the window resampled to fov_size (N, K, f_h, f_w)
         self.resize_to_fov = False
+        # superset: FixedFovealEnv with mask_out merges the last fov_memory (0..16; 0 = off) observations by pixelwise max
+        self.fov_memory = 0
         for k, v in kwargs.items():
             self.__setattr__(k, v)
 
@@ -60,7 +62,8 @@ def _path_from_args(args, num_envs, obs_size, raw_shape, luma, device, host_sour
         sensory_action_space=getattr(args, "sensory_action_space", (0.0, 0.0)),
         peripheral_res=getattr(args, "peripheral_res", None), device=device,
         cache_peripheral=getattr(args, "cache_peripheral", True), side_streams=host_source,
-        antialias=bool(getattr(args, "antialias", True)), **({"channels": channels} if channels != 1 else {}))
+        antialias=bool(getattr(args, "antialias", True)), **({"channels": channels} if channels != 1 else {}),
+        **({"fov_memory": int(args.fov_memory)} if getattr(args, "fov_memory", 0) else {}))
 
 
 class _VecBase(Env):

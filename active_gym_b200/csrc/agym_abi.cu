@@ -559,6 +559,24 @@ int agym_observe_flexible_peripheral(const agym_plan *plan, const uint8_t *d_rin
                                        0, 0, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));
 }
 
+size_t agym_plan_memory_bytes(const agym_plan *plan, int depth) {
+    if (!plan || plan->cfg.fov_h == 0 || depth < 1 || depth > 16) return 0;
+    return static_cast<size_t>(plan->cfg.n_envs) * depth * memory_entry_bytes(plan->dev);
+}
+
+int agym_observe_fixed_memory(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head, const double *d_action,
+                              const uint8_t *d_fov_ctrl, int32_t *d_loc, int depth, uint8_t *d_mem, int32_t *d_mem_loc,
+                              int32_t *d_mem_state, uint8_t *d_out, void *d_out_norm, int norm_dtype, void *stream) {
+    int v = check_fov_args(plan, d_ring, d_head, d_action, d_fov_ctrl, d_loc, d_out);
+    if (v != AGYM_OK) return v;
+    if (depth < 1 || depth > 16 || !d_mem || !d_mem_loc || !d_mem_state) return AGYM_ERR_INVALID_ARG;
+    if (reinterpret_cast<uintptr_t>(d_mem) & 15) return AGYM_ERR_INVALID_ARG;   // entries leave by bulk stores
+    const agym_config &c = plan->cfg;
+    if ((v = check_norm_args(d_out, static_cast<size_t>(c.n_envs) * ring_planes(c) * c.obs_h * c.obs_w, d_out_norm, norm_dtype)) != AGYM_OK) return v;
+    return ret(launch_observe_fixed_memory(plan->dev, d_ring, d_head, d_action, d_fov_ctrl, d_loc, depth, d_mem, d_mem_loc,
+                                           d_mem_state, d_out, d_out_norm, norm_dtype, as_stream(stream)));
+}
+
 int agym_table_cv2(int n_src, int n_dst, int zero_frac_at_border, int32_t *h_s0, int32_t *h_s1, int32_t *h_coef) {
     if (n_src <= 0 || n_dst <= 0 || !h_s0 || !h_s1 || !h_coef) return AGYM_ERR_INVALID_ARG;
     const Cv2Axis ax = build_cv2_axis(n_src, n_dst, zero_frac_at_border != 0);

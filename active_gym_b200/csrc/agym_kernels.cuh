@@ -107,6 +107,11 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
                                     const double *action, const int32_t *atype, const uint8_t *ctrl, int32_t *loc,
                                     int32_t *res, int variant, int pad_h, int pad_w, uint8_t *out, int32_t *err,
                                     void *norm_out, int norm_dt, cudaStream_t st);
+// foveal memory of the fixed fovea (agym_memory.cu): bytes of one entry, and the observe launcher
+size_t memory_entry_bytes(const DevPlan &p);
+cudaError_t launch_observe_fixed_memory(const DevPlan &p, const uint8_t *ring, const int32_t *head, const double *action,
+                                        const uint8_t *ctrl, int32_t *loc, int depth, uint8_t *mem, int32_t *mem_loc,
+                                        int32_t *mem_state, uint8_t *out, void *norm_out, int norm_dt, cudaStream_t st);
 cudaError_t launch_normalize(const uint8_t *src, size_t n, int dtype, void *dst, cudaStream_t st);
 cudaError_t launch_synth(uint8_t *dst, size_t n, uint64_t seed, cudaStream_t st);
 cudaError_t launch_record_step(int n, int is_reset, const double *raw_reward, const uint8_t *done, const uint8_t *reset_mask,

@@ -41,14 +41,18 @@ class ObservationPath:
                  fov_init_loc: Sequence[float] = (0, 0), sensory_action_mode: str = "absolute",
                  sensory_action_space: Sequence[float] = (0.0, 0.0), peripheral_res: Optional[Tuple[int, int]] = None,
                  device: Optional[torch.device] = None, cache_peripheral: bool = True, buffers: Optional[dict] = None,
-                 antialias: bool = True, channels: int = 1):
+                 antialias: bool = True, channels: int = 1, fov_memory: int = 0):
         """``channels``: planes per frame — 1 (grey, the luma of the frames) or 3 (RGB: the channels of DMC renders,
         which must have ``raw_shape == obs_size + (3,)``).  The ring then holds ``frame_stack * channels`` planes
         (``include/agym_b200.h``) and every observation gains a channel axis, ``(N, K, C, h, w)``.
 
         ``antialias``: how the wrappers' ``torchvision.transforms.Resize`` calls (fov_env.py:120, 248, 366-368) are
         restated — antialiased bilinear (the installed torchvision's default, what the fixtures were recorded with) or
-        plain bilinear (the default of older torchvision releases on tensors; SURVEY.md section 8c)."""
+        plain bilinear (the default of older torchvision releases on tensors; SURVEY.md section 8c).
+
+        ``fov_memory``: depth M (1..16) of the fixed fovea's memory (``observe_fixed_memory``), 0 = none.  The path then
+        holds ``mem`` u8 (N, M, E), ``mem_loc`` i32 (N, M, 2) and ``mem_state`` i32 (N, 2), zero = empty
+        (``agym_observe_fixed_memory``), or takes them from ``buffers``."""
         if not torch.cuda.is_available():
             raise RuntimeError("active_gym_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
@@ -63,6 +67,11 @@ class ObservationPath:
         if channels not in (1, 3):
             raise ValueError(f"channels must be 1 (grey) or 3 (RGB), got {channels!r}")
         self.channels = int(channels)
+        if not 0 <= int(fov_memory) <= 16:
+            raise ValueError(f"fov_memory must be within 0..16, got {fov_memory!r}")
+        if fov_memory and self.fov_size is None:
+            raise ValueError("fov_memory needs a fovea (fov_size)")
+        self.fov_memory = int(fov_memory)
         cfg = _lib.Config()
         cfg.n_envs, cfg.frame_stack = self.n_envs, self.frame_stack
         cfg.obs_h, cfg.obs_w = self.obs_size
@@ -107,6 +116,19 @@ class ObservationPath:
                 self.pcache = torch.zeros((N, K) + self.peripheral_res, dtype=torch.float32, device=dev)
             # device error word of the flexible fovea (AGYM_ERR_RES_*): see read_errors()
             self.err = torch.zeros((1,), dtype=torch.int32, device=dev)
+        self.mem = self.mem_loc = self.mem_state = None
+        if self.fov_memory:
+            M = self.fov_memory
+            E = self._L.agym_plan_memory_bytes(self._plan, M) // (N * M)
+            if buffers is not None:
+                self.mem, self.mem_loc, self.mem_state = buffers["mem"], buffers["mem_loc"], buffers["mem_state"]
+                for t, shape in ((self.mem, (N, M, E)), (self.mem_loc, (N, M, 2)), (self.mem_state, (N, 2))):
+                    if tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
+                        raise ValueError("buffers must be contiguous device tensors of this path's shapes")
+            else:
+                self.mem = torch.zeros((N, M, E), dtype=torch.uint8, device=dev)
+                self.mem_loc = torch.zeros((N, M, 2), dtype=torch.int32, device=dev)
+                self.mem_state = torch.zeros((N, 2), dtype=torch.int32, device=dev)
         self._ctrl_reset = torch.full((N,), _lib.FOV_RESET, dtype=torch.uint8, device=dev)
 
     def __del__(self):
@@ -259,6 +281,25 @@ class ObservationPath:
             _lib.check(self._L.agym_observe_fixed(self._plan, _ptr(self.ring), _ptr(self.head), _ptr(act), _ptr(ctrl_t),
                                                   _ptr(self.loc), VARIANTS[variant], _ptr(out), np_, nd, self._stream()),
                        "agym_observe_fixed")
+        return out
+
+    def observe_fixed_memory(self, action, ctrl=None, out: Optional[torch.Tensor] = None,
+                             norm_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The fixed fovea's memory (``agym_observe_fixed_memory``): the fovea update of ``observe_fixed``, a push of the
+        new window unless the env's control is KEEP (RESET empties the memory first), and the pixelwise max of the
+        mask_out frames of the entries held, (N, K, S_h, S_w) or (N, K, 3, S_h, S_w)."""
+        if not self.fov_memory:
+            raise ValueError("observe_fixed_memory needs a path built with fov_memory > 0")
+        ctrl_t = self._ctrl(ctrl)
+        act = None if action is None else self._dev_action(action)
+        if out is None:
+            out = torch.empty(self.out_shape("fixed_memory", "mask"), dtype=torch.uint8, device=self.device)
+        np_, nd = self._norm(out, norm_out)
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.agym_observe_fixed_memory(self._plan, _ptr(self.ring), _ptr(self.head), _ptr(act), _ptr(ctrl_t),
+                                                         _ptr(self.loc), self.fov_memory, _ptr(self.mem), _ptr(self.mem_loc),
+                                                         _ptr(self.mem_state), _ptr(out), np_, nd, self._stream()),
+                       "agym_observe_fixed_memory")
         return out
 
     def observe_peripheral(self, action, ctrl=None, out: Optional[torch.Tensor] = None, use_cache: bool = True,

@@ -171,7 +171,13 @@ class RecordWrapper(Wrapper):
 class FixedFovealEnv(Wrapper):
     """fov_env.py:107-234 for N envs.  Observation: uint8 CUDA tensor (N, K, f_h, f_w), or
     (N, K, S_h, S_w) with ``mask_out`` / ``resize_to_full``; RGB base envs (DMC ``grey=False``) add a channel axis
-    after K, (N, K, 3, h, w)."""
+    after K, (N, K, 3, h, w).
+
+    ``args.fov_memory = M`` (superset, 0..16, default 0 = off; ``mask_out=True`` only): the observation keeps mask_out's
+    shape and is the pixelwise max of the mask_out observations of the env's last min(j, M) fovea updates since its last
+    reset, missing ones counting as zero frames.  A step and a reset push this step's window; envs a masked ``reset``
+    leaves alone push nothing and keep their observation.  The memory follows the fovea's resets only: a life loss inside
+    the base env does not clear it.  ``fov_memory_loc`` / ``fov_memory_count`` expose the state."""
 
     _kind = "fixed"
 
@@ -195,6 +201,16 @@ class FixedFovealEnv(Wrapper):
         self.host_obs = bool(getattr(base, "host_obs", False))
         if self.path.fov_size != self.fov_size:
             raise ValueError("the base env was built from different args (fov_size mismatch)")
+        self.fov_memory = int(getattr(args, "fov_memory", 0) or 0)
+        if not 0 <= self.fov_memory <= 16:
+            raise ValueError(f"fov_memory must be within 0..16, got {self.fov_memory}")
+        if self.fov_memory and self._kind != "fixed":
+            raise ValueError("fov_memory is defined for FixedFovealEnv only (windows of the flexible fovea vary in size, and "
+                             "the peripheral envs have a background)")
+        if self.fov_memory and not self.mask_out:
+            raise ValueError("fov_memory merges mask_out observations: it needs mask_out=True")
+        if self.fov_memory != getattr(self.path, "fov_memory", 0):
+            raise ValueError("the base env was built from different args (fov_memory mismatch)")
         # fov_env.py:125-129 declares Box(low=sas[0], high=sas[1], dtype=int): shape (1,) and, in
         # absolute mode, degenerate.  Kept for compatibility; step() accepts any real (N,2) array.
         self.action_space = Dict({
@@ -245,6 +261,16 @@ class FixedFovealEnv(Wrapper):
     def variant(self) -> str:
         return "mask" if self.mask_out else ("resize_full" if self.resize else "crop")
 
+    @property
+    def fov_memory_loc(self) -> Optional[torch.Tensor]:
+        """(N, M, 2) int32: the fov_loc of each memory slot (``fov_memory_count`` of them are held); None without memory."""
+        return self.path.mem_loc if self.fov_memory else None
+
+    @property
+    def fov_memory_count(self) -> Optional[torch.Tensor]:
+        """(N,) int32: entries the memory of each env holds; None without memory."""
+        return self.path.mem_state[:, 1] if self.fov_memory else None
+
     def _norm_buffer(self):
         if self.obs_dtype is None:
             return None
@@ -252,6 +278,8 @@ class FixedFovealEnv(Wrapper):
         return torch.empty(self.path.out_shape(kind, self.variant), dtype=self.obs_dtype, device=self.path.device)
 
     def _observe(self, action, ctrl, action_type=None, norm_out=None):
+        if self.fov_memory:
+            return self.path.observe_fixed_memory(action, ctrl=ctrl, out=self._out, host_out=self.host_obs, norm_out=norm_out)
         return self.path.observe_fixed(action, variant=self.variant, ctrl=ctrl, out=self._out, host_out=self.host_obs, norm_out=norm_out)
 
     def _run_observe(self, action, ctrl, action_type=None):

@@ -84,7 +84,8 @@ class PipelinedPath:
     def __init__(self, n_envs: int, frame_stack: int, obs_size, raw_shape, shards: int = 1, device=None,
                  luma: Sequence[int] = LUMA_RGB, fov_size=None, fov_init_loc=(0, 0), sensory_action_mode: str = "absolute",
                  sensory_action_space=(0.0, 0.0), peripheral_res=None, cache_peripheral: bool = True,
-                 packed_h2d: bool = True, side_streams: bool = False, antialias: bool = True, channels: int = 1):
+                 packed_h2d: bool = True, side_streams: bool = False, antialias: bool = True, channels: int = 1,
+                 fov_memory: int = 0):
         if not torch.cuda.is_available():
             raise RuntimeError("active_gym_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
@@ -110,6 +111,20 @@ class PipelinedPath:
             if self.peripheral_res and cache_peripheral:
                 self.pcache = torch.zeros((N, K) + self.peripheral_res, dtype=torch.float32, device=dev)
             self.err = torch.zeros((1,), dtype=torch.int32, device=dev)
+            # the fixed fovea's memory (ObservationPath.observe_fixed_memory): one allocation, sliced per shard
+            if not 0 <= int(fov_memory) <= 16:
+                raise ValueError(f"fov_memory must be within 0..16, got {fov_memory!r}")
+            self.fov_memory = int(fov_memory)
+            self.mem = self.mem_loc = self.mem_state = None
+            if self.fov_memory:
+                if self.fov_size is None:
+                    raise ValueError("fov_memory needs a fovea (fov_size)")
+                M, E = self.fov_memory, (K * self.fov_size[0] * self.fov_size[1] + 15) // 16 * 16
+                self.mem = torch.zeros((N, M, E), dtype=torch.uint8, device=dev)
+                self.mem_loc = torch.zeros((N, M, 2), dtype=torch.int32, device=dev)
+                self.mem_state = torch.zeros((N, 2), dtype=torch.int32, device=dev)
+            mem = (lambda lo, hi: dict(mem=self.mem[lo:hi], mem_loc=self.mem_loc[lo:hi], mem_state=self.mem_state[lo:hi])) \
+                if self.fov_memory else (lambda lo, hi: {})
             # RecordWrapper's episode counters (fov_env.py:20-21) live with the rest of the per-env state
             self.ep_len = torch.zeros((N,), dtype=torch.int64, device=dev)
             self.cum_reward = torch.zeros((N,), dtype=torch.float64, device=dev)
@@ -118,9 +133,10 @@ class PipelinedPath:
                                 fov_init_loc=fov_init_loc, sensory_action_mode=sensory_action_mode,
                                 sensory_action_space=sensory_action_space, peripheral_res=peripheral_res, device=dev,
                                 cache_peripheral=cache_peripheral, antialias=antialias, channels=self.channels,
+                                fov_memory=self.fov_memory,
                                 buffers=dict(ring=self.ring[lo:hi], head=self.head[lo:hi], loc=self.loc[lo:hi],
                                              res=self.res[lo:hi], pcache=None if self.pcache is None else self.pcache[lo:hi],
-                                             err=self.err))
+                                             err=self.err, **mem(lo, hi)))
                 for lo, hi in self.ranges]
             # one shard: work is issued on the caller's stream (unless `side_streams`: a host-driven env group keeps its
             # own stream so that two groups overlap each other's copies); several: one side stream each
@@ -401,6 +417,8 @@ class PipelinedPath:
                 p.observe_flexible(a, None if at is None else at[i], variant=variant, ctrl=c, pad=pad, out=out[lo:hi], norm_out=nrm)
             elif kind == "flexible_peripheral":
                 p.observe_flexible_peripheral(a, None if at is None else at[i], ctrl=c, out=out[lo:hi], norm_out=nrm)
+            elif kind == "fixed_memory":
+                p.observe_fixed_memory(a, ctrl=c, out=out[lo:hi], norm_out=nrm)
             else:
                 p.observe_fixed(a, variant=variant, ctrl=c, out=out[lo:hi], norm_out=nrm)
             if host_out:
@@ -419,6 +437,13 @@ class PipelinedPath:
         observations and fov_loc to pinned host memory on the shard streams; returns (out, (h_obs, h_loc, None)),
         valid after ``sync()``."""
         return self._observe("fixed", action, None, variant, ctrl, None, out, host_out, norm_out)
+
+    def observe_fixed_memory(self, action, ctrl=None, out=None, host_out: bool = False, norm_out=None):
+        """The fixed fovea's memory (ObservationPath.observe_fixed_memory) on every shard; ``host_out`` as for
+        ``observe_fixed``."""
+        if not self.fov_memory:
+            raise ValueError("observe_fixed_memory needs a path built with fov_memory > 0")
+        return self._observe("fixed_memory", action, None, "mask", ctrl, None, out, host_out, norm_out)
 
     def observe_peripheral(self, action, ctrl=None, out=None, use_cache: bool = True, host_out: bool = False, norm_out=None):
         """FixedFovealPeripheralEnv._get_fov_state (fov_env.py:375-388), loc update fused."""

@@ -218,6 +218,26 @@ AGYM_API int agym_observe_flexible_peripheral(const agym_plan *plan, const uint8
                           const uint8_t *d_fov_ctrl, int32_t *d_loc, int32_t *d_res, uint8_t *d_out,
                           int32_t *d_err, void *d_out_norm, int norm_dtype, void *stream);
 
+/* Foveal memory of the fixed fovea (a superset of the reference): the observation is the pixelwise max of the mask_out
+ * observations of the env's last min(j, depth) pushes since its last fovea RESET, missing entries counting as zero
+ * frames.  Per env and call, the fovea update of agym_observe_fixed runs first; then d_fov_ctrl decides: RESET empties the
+ * memory and pushes, APPLY pushes, KEEP pushes nothing.  A push stores the (P, f_h, f_w) window after the update and its
+ * loc, evicting the oldest entry once `depth` are held.  With no entry held the output is zero.  The memory follows the
+ * fovea control only: an ingest AGYM_FLAG_HARD_RESET without a fovea RESET leaves it alone.
+ *   d_mem       u8  [N][depth][E], E = round_up(P * f_h * f_w, 16): each entry the packed crop, in the layout
+ *                   agym_observe_fixed(AGYM_OUT_CROP) writes.  Must be 16-byte aligned: the one buffer rejected for its
+ *                   alignment (AGYM_ERR_INVALID_ARG), since the caller sizes it with agym_plan_memory_bytes.
+ *   d_mem_loc   i32 [N][depth][2]: the loc of each entry.
+ *   d_mem_state i32 [N][2]: {newest slot, entries held}; all zeros is an empty memory.
+ * d_out: u8 [N][P][S_h][S_w] at any alignment.  AGYM_ERR_INVALID_ARG for depth outside 1..16, a NULL memory buffer and a
+ * plan without a fovea.  Added without an ABI version bump: the struct and every other signature are unchanged. */
+/* bytes of d_mem for a fovea memory of `depth` entries (1..16) for the plan's N envs (0 when invalid) */
+AGYM_API size_t agym_plan_memory_bytes(const agym_plan *plan, int depth);
+AGYM_API int agym_observe_fixed_memory(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head,
+        const double *d_action, const uint8_t *d_fov_ctrl, int32_t *d_loc, int depth,
+        uint8_t *d_mem, int32_t *d_mem_loc, int32_t *d_mem_state,
+        uint8_t *d_out, void *d_out_norm, int norm_dtype, void *stream);
+
 /* Replaces RecordWrapper's episode counters (fov_env.py:15-67) and the fov_loc / fov_res trace that
  * save_transition keeps when record=True (fov_env.py:152-154, 205-207, 253-256, 332-335), for N envs on the device.
  *   step  (is_reset = 0): ep_len += 1; cum_reward += d_raw_reward (f64 [N], info["raw_reward"]; NULL = 0)

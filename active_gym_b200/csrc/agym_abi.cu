@@ -102,6 +102,8 @@ inline size_t ring_planes(const agym_config &c) { return static_cast<size_t>(c.f
 
 inline cudaStream_t as_stream(void *s) { return reinterpret_cast<cudaStream_t>(s); }
 inline int ret(cudaError_t e) { return e == cudaSuccess ? AGYM_OK : static_cast<int>(e); }
+// launch_observe_flexible: cudaErrorNotSupported = no kernel fits the plan's geometry (nothing was launched)
+inline int ret_flexible(cudaError_t e) { return e == cudaErrorNotSupported ? AGYM_ERR_UNSUPPORTED : ret(e); }
 
 }  // namespace
 
@@ -543,8 +545,8 @@ int agym_observe_flexible(const agym_plan *plan, const uint8_t *d_ring, const in
                           : variant == AGYM_OUT_RESIZE_FOV ? static_cast<size_t>(c.fov_h) * c.fov_w
                                                            : static_cast<size_t>(c.obs_h) * c.obs_w);
     if ((v = check_norm_args(d_out, bytes, d_out_norm, norm_dtype)) != AGYM_OK) return v;
-    return ret(launch_observe_flexible(plan->dev, d_ring, d_head, nullptr, d_action, d_atype, d_fov_ctrl, d_loc, d_res, variant,
-                                       pad_h, pad_w, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));
+    return ret_flexible(launch_observe_flexible(plan->dev, d_ring, d_head, nullptr, d_action, d_atype, d_fov_ctrl, d_loc, d_res,
+                                                variant, pad_h, pad_w, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));
 }
 
 int agym_observe_flexible_peripheral(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head, const float *d_pcache,
@@ -555,8 +557,8 @@ int agym_observe_flexible_peripheral(const agym_plan *plan, const uint8_t *d_rin
     if (plan->cfg.periph_h == 0 || !d_pcache || !d_res) return AGYM_ERR_INVALID_ARG;
     const agym_config &c = plan->cfg;
     if ((v = check_norm_args(d_out, static_cast<size_t>(c.n_envs) * ring_planes(c) * c.obs_h * c.obs_w, d_out_norm, norm_dtype)) != AGYM_OK) return v;
-    return ret(launch_observe_flexible(plan->dev, d_ring, d_head, d_pcache, d_action, d_atype, d_fov_ctrl, d_loc, d_res, kOutPeriph,
-                                       0, 0, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));
+    return ret_flexible(launch_observe_flexible(plan->dev, d_ring, d_head, d_pcache, d_action, d_atype, d_fov_ctrl, d_loc, d_res,
+                                                kOutPeriph, 0, 0, d_out, d_err, d_out_norm, norm_dtype, as_stream(stream)));
 }
 
 size_t agym_plan_memory_bytes(const agym_plan *plan, int depth) {

@@ -403,6 +403,18 @@ cudaError_t set_smem(F func, size_t bytes) {
     return cudaSuccess;
 }
 
+// whether `bytes` of dynamic shared memory fit one block of `func` on the current device: the opt-in limit less the
+// kernel's static shared memory
+template <typename F>
+bool smem_fits(F func, size_t bytes) {
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess ||
+        cudaFuncGetAttributes(&fa, func) != cudaSuccess)
+        return false;
+    return bytes + fa.sharedSizeBytes <= (size_t)optin;
+}
+
 size_t a16(size_t v) { return (v + 15) & ~size_t(15); }
 
 // AGYM_NO_PDL=1: plain stream-ordered launches (A/B comparisons)

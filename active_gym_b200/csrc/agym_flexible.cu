@@ -933,10 +933,12 @@ cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const
             return finish(cudaGetLastError());
         }
     }
-    // window buffers; the peripheral variant adds the background plane and, for generic expand tables, squeeze + W pass
+    // window buffers; the peripheral variant adds the background plane and, for generic expand tables, squeeze + W pass.
+    // Two f32 planes past the shared memory of a block (from about 172 x 172 on a B200): no kernel serves the plan
     const size_t smem = sizeof(float) * 2 * (size_t)p.plane +
                         (periph ? p.plane + sizeof(float) * ((size_t)p.p_h * p.p_w + (size_t)p.p_h * p.S_w) : 0);
 #define AGYM_LAUNCH_FLEX(V)                                                                              \
+    if (!smem_fits(k_observe_flexible<V>, smem)) return cudaErrorNotSupported;                           \
     if ((e = set_smem(k_observe_flexible<V>, smem)) != cudaSuccess) return e;                            \
     k_observe_flexible<V><<<p.N, kThreads, smem, st>>>(q, ring, head, action, atype, ctrl, loc, res, pad_h, pad_w, out, pcache);
     if (periph) { AGYM_LAUNCH_FLEX(kOutPeriph) }

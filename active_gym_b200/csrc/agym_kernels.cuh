@@ -102,6 +102,7 @@ cudaError_t launch_observe_peripheral(const DevPlan &p, const ExpandStd *ew, con
                                       const float *pcache, const double *action, const uint8_t *ctrl, int32_t *loc,
                                       uint8_t *out, void *norm_out, int norm_dt, cudaStream_t st);
 // variant: AGYM_OUT_* or kOutPeriph; pcache: the squeeze cache kOutPeriph expands (null otherwise)
+// cudaErrorNotSupported: no kernel fits the geometry (the generic kernel's two f32 planes exceed a block's shared memory)
 constexpr int kOutPeriph = 4;   // flexible fovea over the peripheral background (agym_observe_flexible_peripheral)
 cudaError_t launch_observe_flexible(const DevPlan &p, const uint8_t *ring, const int32_t *head, const float *pcache,
                                     const double *action, const int32_t *atype, const uint8_t *ctrl, int32_t *loc,

@@ -1040,16 +1040,22 @@ cudaError_t launch_observe_peripheral(const DevPlan &p0, const ExpandStd *ew, co
         const int nw_max = (p.f_w + 3) / 4 + 1;
         const size_t buf_words = (((size_t)p.K * p.p_h * p.p_w + 3) & ~size_t(3)) + (((size_t)p.K * p.f_h * nw_max + 3) & ~size_t(3));
         const size_t fs = 4 * (2 * buf_words + (size_t)p.K * p.p_h * p.S_w) + 8 * ((size_t)p.S_h + 1);
-        int dev = 0, sms = 148, occ = 1;
+        int dev = 0, sms = 148, occ = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        // large peripheries or deep stacks (e.g. 42 x 42 at K = 8) need more shared memory than a block may have:
+        // those plans fall through to the one-CTA-per-env kernel below
 #define AGYM_LAUNCH_PF(KG, PW)                                                                                     \
     {                                                                                                              \
+    if (smem_fits(k_observe_peripheral_v2<KG, PW>, fs)) {                                                          \
         if ((e = set_smem(k_observe_peripheral_v2<KG, PW>, fs)) != cudaSuccess) return e;                          \
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_observe_peripheral_v2<KG, PW>, threads, fs);         \
-        if (occ < 1) return cudaErrorInvalidConfiguration;                                                         \
-        k_observe_peripheral_v2<KG, PW><<<std::min(p.N, sms * occ), threads, fs, st>>>(p, ring, head, pcache, action, \
-                                                                                      ctrl, loc, out, ysegs);     \
+        if (occ >= 1) {                                                                                            \
+            k_observe_peripheral_v2<KG, PW><<<std::min(p.N, sms * occ), threads, fs, st>>>(p, ring, head, pcache, action, \
+                                                                                          ctrl, loc, out, ysegs); \
+            return normalize_after(cudaGetLastError(), out, out_bytes, norm_out, norm_dt, st);                     \
+        }                                                                                                          \
+    }                                                                                                              \
     }
         if (p.K == 4 && p.plane == 7056) AGYM_LAUNCH_PF(4, 1764)
         else if (p.K == 3 && p.plane == 7056) AGYM_LAUNCH_PF(3, 1764)
@@ -1059,7 +1065,6 @@ cudaError_t launch_observe_peripheral(const DevPlan &p0, const ExpandStd *ew, co
         else if (p.K % 2 == 0) AGYM_LAUNCH_PF(2, 0)
         else AGYM_LAUNCH_PF(1, 0)
 #undef AGYM_LAUNCH_PF
-        return normalize_after(cudaGetLastError(), out, out_bytes, norm_out, norm_dt, st);
     }
     if (pcache) {
         if ((e = set_smem(k_observe_peripheral<true>, smem)) != cudaSuccess) return e;

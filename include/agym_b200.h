@@ -194,7 +194,10 @@ AGYM_API int agym_observe_peripheral(const agym_plan *plan, const uint8_t *d_rin
  * Blurred pixels (res rows > fov rows) are within 0.5 LSB + 0.02 of the reference's float value: the W-axis
  * operator runs in 16-bit fixed point (<= 255 * taps / 2^17 LSB from the fp64 weights); windows that the
  * reference does not blur, the mask and the padding are bit exact.
- * d_err (may be NULL): one i32 the kernels OR the AGYM_ERR_RES_* bits into; the caller zeroes and reads it. */
+ * d_err (may be NULL): one i32 the kernels OR the AGYM_ERR_RES_* bits into; the caller zeroes and reads it.
+ * Size limit: a call the fast kernels cannot serve keeps two f32 planes (8 * S_h * S_w bytes) in the shared memory of
+ * one block; past the device's limit (from about 172 x 172 observations on a B200) it returns AGYM_ERR_UNSUPPORTED
+ * and launches nothing.  RESIZE_FULL always takes that kernel. */
 AGYM_API int agym_observe_flexible(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head,
                           const double *d_action, const int32_t *d_atype, const uint8_t *d_fov_ctrl,
                           int32_t *d_loc, int32_t *d_res, int variant, int pad_h, int pad_w,
@@ -211,6 +214,8 @@ AGYM_API int agym_observe_flexible(const agym_plan *plan, const uint8_t *d_ring,
  * blurred, within 0.5 LSB + 0.02 of the reference's float value when blurred); background pixels are within 0.5 LSB +
  * 0.01 of it, and bit for bit agym_observe_peripheral's where that call runs its standard-geometry kernel (grey, 84x84
  * observations, 20x20 periphery).  Any d_out alignment is served (the fast kernel needs 16 bytes).
+ * Size limit as for agym_observe_flexible, the table-driven kernel adding the background plane, the squeeze and its W
+ * pass (S_h * S_w + 4 * p_h * (p_w + S_w) bytes): AGYM_ERR_UNSUPPORTED past it.
  * AGYM_ERR_INVALID_ARG for a plan without a fovea or a periphery and for NULL d_pcache or d_res.  Added without an ABI
  * version bump: the struct and every other signature are unchanged. */
 AGYM_API int agym_observe_flexible_peripheral(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head,

@@ -22,6 +22,7 @@ OUT_CROP, OUT_MASK, OUT_RESIZE_FULL, OUT_RESIZE_FOV = 0, 1, 2, 3
 ATYPE_FOV_LOC, ATYPE_FOV_RES = 0, 1
 ERR_RES_RANGE, ERR_RES_FRACTION = 1, 2
 DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
+BG_ZERO, BG_PERIPHERY = 0, 1
 
 # the symbols include/agym_b200.h declares; tests check that the .so exports every one
 EXPORTS = (
@@ -30,6 +31,7 @@ EXPORTS = (
     "agym_stack", "agym_observe_fixed", "agym_observe_peripheral", "agym_observe_flexible",
     "agym_synth_frames", "agym_table_cv2", "agym_table_aa", "agym_table_blur", "agym_normalize", "agym_plan_used_rows", "agym_ingest_atari_packed", "agym_record_step",
     "agym_observe_flexible_peripheral", "agym_plan_memory_bytes", "agym_observe_fixed_memory",
+    "agym_observe_fixed_memory_paste",
 )
 
 
@@ -78,6 +80,7 @@ def lib() -> C.CDLL:
     L.agym_plan_memory_bytes.restype = sz
     L.agym_plan_memory_bytes.argtypes = [vp, i32]
     L.agym_observe_fixed_memory.argtypes = [vp] * 6 + [i32] + [vp] * 5 + [i32, vp]
+    L.agym_observe_fixed_memory_paste.argtypes = [vp] * 7 + [i32, i32] + [vp] * 5 + [i32, vp]
     L.agym_record_step.argtypes = [i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.agym_synth_frames.argtypes = [vp, sz, u64, vp]
     L.agym_normalize.argtypes = [vp, sz, i32, vp, vp]

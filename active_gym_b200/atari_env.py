@@ -39,6 +39,9 @@ class AtariEnvArgs:
         self.resize_to_fov = False
         # superset: FixedFovealEnv with mask_out merges the last fov_memory (0..16; 0 = off) observations by pixelwise max
         self.fov_memory = 0
+        # superset: how the memory merges its windows — "max" (pixelwise max of the mask_out observations) or "paste"
+        # (the windows laid oldest to newest over the background: zeros, or the periphery of FixedFovealPeripheralEnv)
+        self.fov_memory_merge = "max"
         for k, v in kwargs.items():
             self.__setattr__(k, v)
 

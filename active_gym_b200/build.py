@@ -15,7 +15,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "lib", "libagym_b200.so")
-SOURCES = ["agym_ingest.cu", "agym_ingest_std.cu", "agym_observe.cu", "agym_flexible.cu", "agym_memory.cu", "agym_misc.cu", "agym_abi.cu", "agym_tables.cpp"]
+SOURCES = ["agym_ingest.cu", "agym_ingest_std.cu", "agym_observe.cu", "agym_flexible.cu", "agym_memory.cu", "agym_memory_paste.cu", "agym_misc.cu", "agym_abi.cu", "agym_tables.cpp"]
 HEADERS = ["agym_kernels.cuh", "agym_device.cuh", "agym_tables.h", os.path.join("..", "..", "include", "agym_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -113,6 +113,12 @@ size_t memory_entry_bytes(const DevPlan &p);
 cudaError_t launch_observe_fixed_memory(const DevPlan &p, const uint8_t *ring, const int32_t *head, const double *action,
                                         const uint8_t *ctrl, int32_t *loc, int depth, uint8_t *mem, int32_t *mem_loc,
                                         int32_t *mem_state, uint8_t *out, void *norm_out, int norm_dt, cudaStream_t st);
+// the same memory pasted newest-on-top over a background (agym_memory_paste.cu); background: AGYM_BG_*, pcache only for
+// AGYM_BG_PERIPHERY; cudaErrorNotSupported: the plane and the periphery do not fit one block's shared memory
+cudaError_t launch_observe_memory_paste(const DevPlan &p, const uint8_t *ring, const int32_t *head, const float *pcache,
+                                        const double *action, const uint8_t *ctrl, int32_t *loc, int depth, int background,
+                                        uint8_t *mem, int32_t *mem_loc, int32_t *mem_state, uint8_t *out, void *norm_out,
+                                        int norm_dt, cudaStream_t st);
 cudaError_t launch_normalize(const uint8_t *src, size_t n, int dtype, void *dst, cudaStream_t st);
 cudaError_t launch_synth(uint8_t *dst, size_t n, uint64_t seed, cudaStream_t st);
 cudaError_t launch_record_step(int n, int is_reset, const double *raw_reward, const uint8_t *done, const uint8_t *reset_mask,

@@ -23,7 +23,7 @@ from .spaces import Box
 
 
 class DMCEnvArgs:
-    """Source-compatible with dmc_env.py:56-76 (+ ``resize_to_full``, ``resize_to_fov`` and ``fov_memory`` defaults, see AtariEnvArgs)."""
+    """Source-compatible with dmc_env.py:56-76 (+ ``resize_to_full``, ``resize_to_fov``, ``fov_memory`` and ``fov_memory_merge`` defaults, see AtariEnvArgs)."""
 
     def __init__(self, domain_name: str, task_name: str, seed: int, obs_size: Tuple[int, int], **kwargs):
         self.env_backend = "dmc"
@@ -45,6 +45,7 @@ class DMCEnvArgs:
         self.resize_to_full = False
         self.resize_to_fov = False
         self.fov_memory = 0
+        self.fov_memory_merge = "max"
         for k, v in kwargs.items():
             self.__setattr__(k, v)
 

@@ -302,6 +302,33 @@ class ObservationPath:
                        "agym_observe_fixed_memory")
         return out
 
+    _BACKGROUNDS = {"zero": _lib.BG_ZERO, "periphery": _lib.BG_PERIPHERY}
+
+    def observe_memory_paste(self, action, ctrl=None, background: str = "zero", out: Optional[torch.Tensor] = None,
+                             norm_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The fixed fovea's memory merged by pasting (``agym_observe_fixed_memory_paste``): the fovea and memory update
+        of ``observe_fixed_memory`` (same buffers, same bytes), then per plane the background — ``"zero"``, or
+        ``"periphery"``: ``observe_peripheral``'s blurred periphery of the current ring, from the squeeze cache — with
+        the held windows written over it oldest to newest, (N, K, S_h, S_w) or (N, K, 3, S_h, S_w)."""
+        if not self.fov_memory:
+            raise ValueError("observe_memory_paste needs a path built with fov_memory > 0")
+        if background not in self._BACKGROUNDS:
+            raise ValueError(f"background must be 'zero' or 'periphery', got {background!r}")
+        if background == "periphery" and self.pcache is None:
+            raise ValueError("the periphery background needs the squeeze cache: build the path with peripheral_res and "
+                             "cache_peripheral=True")
+        ctrl_t = self._ctrl(ctrl)
+        act = None if action is None else self._dev_action(action)
+        if out is None:
+            out = torch.empty(self.out_shape("fixed_memory", "mask"), dtype=torch.uint8, device=self.device)
+        np_, nd = self._norm(out, norm_out)
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.agym_observe_fixed_memory_paste(
+                self._plan, _ptr(self.ring), _ptr(self.head), _ptr(self.pcache), _ptr(act), _ptr(ctrl_t), _ptr(self.loc),
+                self.fov_memory, self._BACKGROUNDS[background], _ptr(self.mem), _ptr(self.mem_loc), _ptr(self.mem_state),
+                _ptr(out), np_, nd, self._stream()), "agym_observe_fixed_memory_paste")
+        return out
+
     def observe_peripheral(self, action, ctrl=None, out: Optional[torch.Tensor] = None, use_cache: bool = True,
                            norm_out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """FixedFovealPeripheralEnv._get_fov_state (fov_env.py:375-388), loc update fused."""

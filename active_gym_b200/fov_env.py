@@ -177,7 +177,12 @@ class FixedFovealEnv(Wrapper):
     shape and is the pixelwise max of the mask_out observations of the env's last min(j, M) fovea updates since its last
     reset, missing ones counting as zero frames.  A step and a reset push this step's window; envs a masked ``reset``
     leaves alone push nothing and keep their observation.  The memory follows the fovea's resets only: a life loss inside
-    the base env does not clear it.  ``fov_memory_loc`` / ``fov_memory_count`` expose the state."""
+    the base env does not clear it.  ``fov_memory_loc`` / ``fov_memory_count`` expose the state.
+
+    ``args.fov_memory_merge`` (superset, ``"max"`` by default) selects how the held windows merge.  ``"paste"`` lays them
+    over a zero background from the oldest to the newest, so at each pixel the newest window covering it wins (a bright
+    sprite that moved away does not linger over the fresh view of its old place).  The memory, its state and the rules
+    above are the same under both; other values raise ``ValueError``."""
 
     _kind = "fixed"
 
@@ -204,10 +209,20 @@ class FixedFovealEnv(Wrapper):
         self.fov_memory = int(getattr(args, "fov_memory", 0) or 0)
         if not 0 <= self.fov_memory <= 16:
             raise ValueError(f"fov_memory must be within 0..16, got {self.fov_memory}")
-        if self.fov_memory and self._kind != "fixed":
-            raise ValueError("fov_memory is defined for FixedFovealEnv only (windows of the flexible fovea vary in size, and "
-                             "the peripheral envs have a background)")
-        if self.fov_memory and not self.mask_out:
+        self.fov_memory_merge = getattr(args, "fov_memory_merge", "max")
+        if self.fov_memory_merge not in ("max", "paste"):
+            raise ValueError(f"fov_memory_merge must be 'max' or 'paste', got {self.fov_memory_merge!r}")
+        if self.fov_memory and self._kind == "peripheral":
+            if self.fov_memory_merge != "paste":
+                raise ValueError("fov_memory on FixedFovealPeripheralEnv needs fov_memory_merge=\"paste\": a max over the "
+                                 "blurred backgrounds of past frames is not a useful observation")
+            if self.path.pcache is None:
+                raise ValueError("fov_memory on FixedFovealPeripheralEnv pastes over the squeeze cache: build the base env "
+                                 "with cache_peripheral=True")
+        elif self.fov_memory and self._kind != "fixed":
+            raise ValueError("fov_memory is defined for FixedFovealEnv and FixedFovealPeripheralEnv only (windows of the "
+                             "flexible fovea vary in size)")
+        elif self.fov_memory and not self.mask_out:
             raise ValueError("fov_memory merges mask_out observations: it needs mask_out=True")
         if self.fov_memory != getattr(self.path, "fov_memory", 0):
             raise ValueError("the base env was built from different args (fov_memory mismatch)")
@@ -277,9 +292,16 @@ class FixedFovealEnv(Wrapper):
         kind = "peripheral" if self._kind == "peripheral" else self._kind
         return torch.empty(self.path.out_shape(kind, self.variant), dtype=self.obs_dtype, device=self.path.device)
 
+    def _observe_memory(self, action, ctrl, norm_out):
+        if self.fov_memory_merge == "paste":
+            bg = "periphery" if self._kind == "peripheral" else "zero"
+            return self.path.observe_memory_paste(action, ctrl=ctrl, background=bg, out=self._out, host_out=self.host_obs,
+                                                  norm_out=norm_out)
+        return self.path.observe_fixed_memory(action, ctrl=ctrl, out=self._out, host_out=self.host_obs, norm_out=norm_out)
+
     def _observe(self, action, ctrl, action_type=None, norm_out=None):
         if self.fov_memory:
-            return self.path.observe_fixed_memory(action, ctrl=ctrl, out=self._out, host_out=self.host_obs, norm_out=norm_out)
+            return self._observe_memory(action, ctrl, norm_out)
         return self.path.observe_fixed(action, variant=self.variant, ctrl=ctrl, out=self._out, host_out=self.host_obs, norm_out=norm_out)
 
     def _run_observe(self, action, ctrl, action_type=None):
@@ -433,7 +455,13 @@ class FlexibleFovealEnv(FixedFovealEnv):
 
 class FixedFovealPeripheralEnv(FixedFovealEnv):
     """fov_env.py:358-388 for N envs: blurred periphery (squeeze to ``peripheral_res``, expand
-    back) with the full-resolution fovea pasted at ``fov_loc``; (N, K, S_h, S_w) uint8."""
+    back) with the full-resolution fovea pasted at ``fov_loc``; (N, K, S_h, S_w) uint8.
+
+    ``args.fov_memory = M`` (superset, 1..16) needs ``fov_memory_merge="paste"`` and the squeeze cache
+    (``cache_peripheral=True``); either missing raises ``ValueError``.  The observation is then the periphery of the current
+    frames with the env's last min(j, M) windows since its last fovea reset pasted over it from the oldest to the newest,
+    the newest being this step's fovea; ``args.mask_out`` is ignored, as the reference's constructor forces it off.  Pushes,
+    resets, ``fov_memory_loc`` and ``fov_memory_count`` are FixedFovealEnv's."""
 
     _kind = "peripheral"
 
@@ -447,6 +475,8 @@ class FixedFovealPeripheralEnv(FixedFovealEnv):
             raise ValueError("the base env was built from different args (peripheral_res mismatch)")
 
     def _observe(self, action, ctrl, action_type=None, norm_out=None):
+        if self.fov_memory:
+            return self._observe_memory(action, ctrl, norm_out)
         return self.path.observe_peripheral(action, ctrl=ctrl, out=self._out, host_out=self.host_obs, norm_out=norm_out)
 
 

@@ -381,7 +381,8 @@ class PipelinedPath:
         self.join()
         return out.view(self.stack_shape)
 
-    def _observe(self, kind: str, action, action_type, variant: str, ctrl, pad, out, host_out: bool, norm_out=None):
+    def _observe(self, kind: str, action, action_type, variant: str, ctrl, pad, out, host_out: bool, norm_out=None,
+                 background=None):
         shape = self.out_shape(kind, variant, pad)
         if norm_out is not None and tuple(norm_out.shape) != tuple(shape):
             raise ValueError(f"norm_out must have the observation's shape {tuple(shape)}")
@@ -419,6 +420,8 @@ class PipelinedPath:
                 p.observe_flexible_peripheral(a, None if at is None else at[i], ctrl=c, out=out[lo:hi], norm_out=nrm)
             elif kind == "fixed_memory":
                 p.observe_fixed_memory(a, ctrl=c, out=out[lo:hi], norm_out=nrm)
+            elif kind == "memory_paste":
+                p.observe_memory_paste(a, ctrl=c, background=background, out=out[lo:hi], norm_out=nrm)
             else:
                 p.observe_fixed(a, variant=variant, ctrl=c, out=out[lo:hi], norm_out=nrm)
             if host_out:
@@ -444,6 +447,16 @@ class PipelinedPath:
         if not self.fov_memory:
             raise ValueError("observe_fixed_memory needs a path built with fov_memory > 0")
         return self._observe("fixed_memory", action, None, "mask", ctrl, None, out, host_out, norm_out)
+
+    def observe_memory_paste(self, action, ctrl=None, background: str = "zero", out=None, host_out: bool = False,
+                             norm_out=None):
+        """The fixed fovea's memory merged by pasting (ObservationPath.observe_memory_paste) on every shard;
+        ``host_out`` as for ``observe_fixed``."""
+        if not self.fov_memory:
+            raise ValueError("observe_memory_paste needs a path built with fov_memory > 0")
+        if background == "periphery" and self.pcache is None:
+            raise ValueError("the periphery background needs the squeeze cache: build with cache_peripheral=True")
+        return self._observe("memory_paste", action, None, "mask", ctrl, None, out, host_out, norm_out, background=background)
 
     def observe_peripheral(self, action, ctrl=None, out=None, use_cache: bool = True, host_out: bool = False, norm_out=None):
         """FixedFovealPeripheralEnv._get_fov_state (fov_env.py:375-388), loc update fused."""

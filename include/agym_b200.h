@@ -243,6 +243,28 @@ AGYM_API int agym_observe_fixed_memory(const agym_plan *plan, const uint8_t *d_r
         uint8_t *d_mem, int32_t *d_mem_loc, int32_t *d_mem_state,
         uint8_t *d_out, void *d_out_norm, int norm_dtype, void *stream);
 
+/* The same memory merged by pasting instead of by max (a superset of the reference): per plane, the background, then
+ * the held windows written over it from the oldest to the newest, so at every pixel the newest window that covers it
+ * wins.  With no entry held the output is the background alone.  The fovea update and the memory update (RESET empties
+ * and pushes, APPLY pushes, KEEP pushes nothing) are agym_observe_fixed_memory's: d_mem, d_mem_loc and d_mem_state have
+ * its layout and sizing (agym_plan_memory_bytes), and after the same sequence of calls hold the same bytes under either
+ * merge.
+ *   background AGYM_BG_ZERO: zeros; with depth 1 and every call pushing this is agym_observe_fixed(AGYM_OUT_MASK).
+ *   background AGYM_BG_PERIPHERY: Resize(S)(Resize(p)(plane)) of the CURRENT ring (fov_env.py:366-368, 376), expanded
+ *              from d_pcache; with depth 1 and every call pushing this is agym_observe_peripheral.  Its pixels are bit
+ *              for bit agym_observe_peripheral's where that call runs its standard-geometry kernel (grey, 84x84, 20x20),
+ *              and within 0.5 LSB + 0.01 of the reference's float value elsewhere.  Pasted pixels are exact.
+ * d_pcache is ignored under AGYM_BG_ZERO.  d_out: u8 [N][P][S_h][S_w] at any alignment.  AGYM_ERR_INVALID_ARG for a
+ * depth outside 1..16, a NULL memory buffer, a d_mem that is not 16-byte aligned, a plan without a fovea, an unknown
+ * background, and AGYM_BG_PERIPHERY with a NULL d_pcache or a plan without a periphery.  AGYM_ERR_UNSUPPORTED when the
+ * plane and the periphery do not fit one block's shared memory.  Added without an ABI version bump. */
+#define AGYM_BG_ZERO 0        /* background of the pasted memory: zeros (mask_out)                 */
+#define AGYM_BG_PERIPHERY 1   /* Resize(S)(Resize(p)(plane)) of the current ring, from d_pcache    */
+AGYM_API int agym_observe_fixed_memory_paste(const agym_plan *plan, const uint8_t *d_ring, const int32_t *d_head,
+        const float *d_pcache, const double *d_action, const uint8_t *d_fov_ctrl, int32_t *d_loc, int depth,
+        int background, uint8_t *d_mem, int32_t *d_mem_loc, int32_t *d_mem_state,
+        uint8_t *d_out, void *d_out_norm, int norm_dtype, void *stream);
+
 /* Replaces RecordWrapper's episode counters (fov_env.py:15-67) and the fov_loc / fov_res trace that
  * save_transition keeps when record=True (fov_env.py:152-154, 205-207, 253-256, 332-335), for N envs on the device.
  *   step  (is_reset = 0): ep_len += 1; cum_reward += d_raw_reward (f64 [N], info["raw_reward"]; NULL = 0)
